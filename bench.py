@@ -6,6 +6,7 @@ tokens, random-init weights.
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 --master-port 29511 \
         bench.py --gpus 8 --steps 8 --warmup 3
     python bench.py --impl reference ...        # the UNMODIFIED reference (baseline/_ref) on the same config
+    python bench.py --steps 8 --dump-outputs out/  # also write what the last timed step computed (out/*.npy)
 
 A "step" is one inner optimizer step of every worker: ``batch`` sequences x ``seq`` tokens per worker processed as
 ``batch / micro_batch`` gradient-accumulated micro-batches, global-norm clip, AdamW, LR schedule; the DiLoCo outer step
@@ -45,7 +46,15 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--compression", default=None)
     ap.add_argument("--no-fused-collective", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the loss of the last timed step and a fixed sample of the fp32 master "
+                         "weights it left behind as DIR/<name>.npy, so that two builds can be compared output for output")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return a
 
 
 # --------------------------------------------------------------------------------------------------- clocks
@@ -94,6 +103,24 @@ class ClockSampler:
                     reasons.add(name)
         return {"sm_mhz": statistics.median(sm) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "power_w_max": max(pw) if pw else None, "samples": len(sm), "reasons": sorted(reasons)}
+
+
+DUMP_PARAM_SAMPLE = 1 << 23          # 32 MB of fp32 weights
+
+
+def dump_outputs(out_dir: str, loss, master) -> None:
+    """What a caller of ``train_step`` holds after the last timed step: the loss it returned and the parameters it left.
+    Models larger than DUMP_PARAM_SAMPLE parameters are sampled at fixed (seed 0) positions of the flat master vector."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    n = master.numel()
+    if n > DUMP_PARAM_SAMPLE:
+        idx = torch.randint(n, (DUMP_PARAM_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+        master = master[idx.to(master.device)]
+    np.save(os.path.join(out_dir, "loss.npy"), loss.detach().float().reshape(1).cpu().numpy())
+    np.save(os.path.join(out_dir, "master_params.npy"), master.detach().float().cpu().numpy())
 
 
 def baseline_number():
@@ -178,7 +205,7 @@ def run_ours(a) -> dict:
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
     for _ in range(a.steps):
-        tr.train_step(it)
+        loss = tr.train_step(it)
     ev1.record()
     sync()
     my_ms = ev0.elapsed_time(ev1)
@@ -191,6 +218,8 @@ def run_ours(a) -> dict:
         per_rank_ms = [round(float(x.item()), 3) for x in allt]
     launches = _lib.launch_count()
     clocks = sampler.stop()
+    if a.dump_outputs and rank == 0:        # before the outer-sync timing and the e2e arm move the weights on
+        dump_outputs(a.dump_outputs, loss, model.arena.master)
     outer_in_window = sum(1 for s in range(a.warmup + 1, a.warmup + a.steps + 1) if s % H == 0)
     value = tokens_per_step * a.steps / (dev_ms / 1e3)
 

@@ -24,5 +24,28 @@ def pytest_collection_modifyitems(config, items):
 
 
 @pytest.fixture(scope="session")
-def ref_model_dir():
-    return "/root/reference/tests/models/llama-2m-fresh" if os.path.isdir("/root/reference/tests/models/llama-2m-fresh") else None
+def ref_model_dir(tmp_path_factory):
+    """The reference's 2M-parameter test checkpoint (tests/models/llama-2m-fresh there), rebuilt from
+    tests/golden/llama-2m-fresh.  Its config files and safetensors header are stored verbatim; the 1 MB of fresh-init
+    weights are redrawn the way HF initialises them (norm weights 1, matrices N(0, 0.02)) from a fixed numpy seed."""
+    import json
+    import shutil
+    import struct
+
+    import numpy as np
+
+    src = os.path.join(ROOT, "tests", "golden", "llama-2m-fresh")
+    dst = tmp_path_factory.mktemp("llama-2m-fresh")
+    for name in ("config.json", "generation_config.json"):
+        shutil.copy(os.path.join(src, name), dst / name)
+    with open(os.path.join(src, "model.safetensors.header.json"), "rb") as f:
+        header = f.read()
+    tensors = sorted((v["data_offsets"], v["shape"]) for k, v in json.loads(header).items() if k != "__metadata__")
+    rng = np.random.default_rng(0)
+    data = bytearray()
+    for (begin, end), shape in tensors:
+        assert begin == len(data) and end - begin == 4 * int(np.prod(shape))
+        w = np.ones(shape, np.float32) if len(shape) == 1 else rng.normal(0.0, 0.02, shape).astype(np.float32)
+        data += w.astype("<f4").tobytes()
+    (dst / "model.safetensors").write_bytes(struct.pack("<Q", len(header)) + header + bytes(data))
+    return str(dst)

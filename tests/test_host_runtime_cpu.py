@@ -24,11 +24,10 @@ def test_safetensors_roundtrip(tmp_path):
 
 @needs_host
 def test_native_safetensors_matches_python_and_validates(tmp_path, ref_model_dir):
-    if ref_model_dir is not None:
-        path = os.path.join(ref_model_dir, "model.safetensors")
-        a = st._load_native(path)
-        header, base = st.read_header(path)
-        assert len(a) == 21 and set(a) == {k for k in header if k != "__metadata__"}
+    path = os.path.join(ref_model_dir, "model.safetensors")
+    a = st._load_native(path)
+    header, base = st.read_header(path)
+    assert len(a) == 21 and set(a) == {k for k in header if k != "__metadata__"}
     bad = tmp_path / "bad.safetensors"
     bad.write_bytes(b"\x10\x00\x00\x00\x00\x00\x00\x00" + b'{"x":{"dtype":"F32","shape":[4],"data_offsets":[0,16]}}'[:16])
     with pytest.raises(ValueError):

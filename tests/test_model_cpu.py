@@ -1,8 +1,13 @@
 """Model parity on CPU: our hand-scheduled engine vs HF LlamaForCausalLM (the model the reference trains)."""
+import os
+
+import numpy as np
 import pytest
 import torch
 
 from opendiloco_b200 import LlamaConfig, LlamaForCausalLM
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def _hf():
@@ -10,12 +15,8 @@ def _hf():
     return tr
 
 
-def test_matches_hf_llama_fp32(ref_model_dir, tmp_path):
+def test_matches_hf_llama_fp32(ref_model_dir):
     tr = _hf()
-    if ref_model_dir is None:
-        cfg = LlamaConfig(hidden_size=64, intermediate_size=256, num_hidden_layers=2, num_attention_heads=2, vocab_size=1024)
-        LlamaForCausalLM(cfg, precision="32-true", seed=1).save_pretrained(str(tmp_path))
-        ref_model_dir = str(tmp_path)
     torch.manual_seed(0)
     ours = LlamaForCausalLM.from_pretrained(ref_model_dir, precision="32-true")
     hf = tr.LlamaForCausalLM.from_pretrained(ref_model_dir, attn_implementation="sdpa").float()
@@ -28,6 +29,21 @@ def test_matches_hf_llama_fp32(ref_model_dir, tmp_path):
     for n, p in ours.named_parameters():
         assert torch.allclose(p.grad, hfp[n].grad, atol=2e-6, rtol=1e-4), n
     assert list(ours.state_dict().keys()) == list(hf.state_dict().keys())
+
+
+def test_matches_stored_hf_outputs(ref_model_dir):
+    """Loss and a fixed sample of the gradients HF LlamaForCausalLM computed on the reference's 2M checkpoint (fp32, sdpa,
+    CPU; tests/golden/llama-2m-fresh/hf_outputs.npz), so the parity check does not depend on transformers being installed."""
+    gold = np.load(os.path.join(GOLDEN, "llama-2m-fresh", "hf_outputs.npz"))
+    ours = LlamaForCausalLM.from_pretrained(ref_model_dir, precision="32-true")
+    ours.train()
+    ids = torch.from_numpy(gold["input_ids"])
+    loss = ours(input_ids=ids, labels=ids).loss
+    assert abs(loss.item() - float(gold["loss"])) < 1e-5
+    loss.backward()
+    for n, p in ours.named_parameters():
+        got = p.grad.reshape(-1)[torch.from_numpy(gold[f"index:{n}"]).long()]
+        assert torch.allclose(got, torch.from_numpy(gold[f"grad:{n}"]), atol=2e-6, rtol=1e-4), n
 
 
 def test_gqa_matches_hf(tmp_path):

@@ -202,8 +202,15 @@ def test_run_training_sh_launches_two_workers(tmp_path):
     """The launcher contract of the reference (open_diloco/run_training.sh:28-36): ``./run_training.sh <N> <gpus per worker>
     <initial_peer|auto> [train_fsdp flags]`` starts N separate torchrun jobs that meet on one rendezvous address, each logging
     to logs/log<i>.  Two CPU workers, 4 steps, one outer step."""
+    # The launcher gives worker i the GPU slice "i"; with one GPU that puts worker 0 on NCCL and worker 1, which sees no GPU,
+    # on gloo, and the two never meet.  A ``torchrun`` first on PATH records the slice and hides the GPUs from the workers.
+    shim = tmp_path / "bin" / "torchrun"
+    shim.parent.mkdir()
+    shim.write_text('#!/bin/sh\necho "launcher slice: CUDA_VISIBLE_DEVICES=$CUDA_VISIBLE_DEVICES"\n'
+                    f'export CUDA_VISIBLE_DEVICES=\nexec "{sys.executable}" -m torch.distributed.run "$@"\n')
+    shim.chmod(0o755)
     env = dict(os.environ, PYTHONPATH=ROOT, CUDA_VISIBLE_DEVICES="", OMP_NUM_THREADS="2", WANDB_MODE="disabled", DILOCO_WAIT="1",
-               DILOCO_PORT=str(free_port()))
+               DILOCO_PORT=str(free_port()), PATH=f"{shim.parent}{os.pathsep}{os.environ.get('PATH', '')}")
     args = [a for a in BASE if a != "16"]          # drop the DP total batch; DiLoCo: per-worker batch
     args[args.index("--total_batch_size"):args.index("--total_batch_size") + 1] = ["--total_batch_size", "4"]
     cmd = ["bash", os.path.join(ROOT, "run_training.sh"), "2", "1", "auto", *args, "--hv.local_steps", "2", "--max_steps", "4",
@@ -212,6 +219,7 @@ def test_run_training_sh_launches_two_workers(tmp_path):
     logs = {i: open(f"{tmp_path}/logs/log{i}").read() for i in (0, 1)}
     assert res.returncode == 0, res.stdout[-1500:] + res.stderr[-1500:] + logs[0][-2000:] + logs[1][-1500:]
     assert "Training completed." in logs[0] and "Training completed." in logs[1]
+    assert all(f"launcher slice: CUDA_VISIBLE_DEVICES={i}\n" in logs[i] for i in (0, 1))
     assert "DiLoCo enabled: 2 workers x 1 GPU(s)" in logs[0]
     assert set(_load(f"{tmp_path}/log.pkl")) == {1, 2, 3, 4}
 
