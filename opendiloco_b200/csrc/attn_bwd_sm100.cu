@@ -20,6 +20,10 @@
 // dV [256,320) dK [320,384) dQ [384,448).   512 threads in four warpgroups with their own register budgets (setmaxnreg):
 // warp 0 TMA + warp 1 MMA (96 regs), warps 4-11 element-wise (two threads per KEY row, 64 queries each; 160 regs) +
 // dK/dV epilogue, warps 12-15 dQ drain (TMEM -> staging -> TMA reduce-add; 96 regs).
+//
+// MASKED instantiation (padding / per-document masks, see odb_attn_mask_prep in attn_sm100.cu): key tile kt visits query
+// tiles kt .. q_hi[b, kt]; the per-query-tile statistics block carries a third row, lo of the 128 queries, so an
+// element-wise thread (one key row) applies allowed(s, t) = t == s || (lo[s] <= t < s && valid[t]) when its warp needs it.
 #include "common.cuh"
 #include "sm100_ptx.cuh"
 #include "packed_math.cuh"
@@ -45,8 +49,10 @@ template <int EWS> struct Roles {
 };
 constexpr int QST = 3;                         // Q / dO / stats pipeline stages
 constexpr int STAT_BYTES = 2 * 128 * 4;        // per (b, h, query tile): -lse*log2(e) [128] then -D*scale [128]
+constexpr int MASKED_STAT_BYTES = 3 * 128 * 4; // ... then lo [128] (int32) of the MASKED instantiation
 // K, V, QST x (Q, dO), dS^T (2 query chunks), dQ staging fp32 [128 x 64] = 2 chunks of 128 B rows, stats, barriers
 constexpr int SMEM_BYTES = 2 * TILE + 2 * QST * TILE + 2 * TILE + 2 * TILE + QST * STAT_BYTES + 1024 + 256;
+constexpr int MASKED_SMEM_BYTES = SMEM_BYTES + QST * (MASKED_STAT_BYTES - STAT_BYTES);
 constexpr uint32_t TMEM_COLS = 512;
 constexpr int DEFAULT_EWS = 2;
 
@@ -55,6 +61,10 @@ struct Params {
   float scale, scale_log2;
   const float* stats;    // [B, Hq, S/128, 2, 128] written by the pre-pass
   long long* dbg;        // optional timeline of CTA (0,0,0): [iteration][16] clock64 stamps (nullptr = off)
+  // MASKED only (odb_attn_mask_prep outputs)
+  const uint32_t* vbits; // [B, S/32] key-valid bits
+  const int* q_hi;       // [B, S/128] last query tile a key tile visits
+  const int* lo_hi;      // [B, S/128] largest lo of a query tile
 };
 
 #define BWD_STAMP(slot) do { if (dbg_on) p.dbg[it * 16 + (slot)] = clock64(); } while (0)
@@ -90,12 +100,13 @@ __device__ __forceinline__ void tmem_st_cols(uint32_t taddr, const uint32_t (&r)
   else tmem_st_32x32b_x32(taddr, r);
 }
 
-template <int EWS>
+template <int EWS, bool MASKED = false>
 __global__ void __launch_bounds__(Roles<EWS>::THREADS, 1)
 attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_constant__ CUtensorMap tmap_do,
                 const __grid_constant__ CUtensorMap tmap_dq, const __grid_constant__ CUtensorMap tmap_dk,
                 const __grid_constant__ CUtensorMap tmap_dv, Params p) {
   using R = Roles<EWS>;
+  constexpr int SB = MASKED ? MASKED_STAT_BYTES : STAT_BYTES, SF = SB / 4;   // statistics block: bytes / floats
   constexpr int EW_THREADS = R::EW_THREADS, DRAIN_WARP0 = R::DRAIN_WARP0, NQ = R::NQ, DC = R::DC;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -106,7 +117,7 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
   uint8_t* sdS = sdO + QST * TILE;         // dS^T: [2 query-chunks][128 key rows][128 B]  (also the dK/dV store staging)
   uint8_t* sdQ = sdS + 2 * TILE;           // fp32 staging: [2 column-chunks][128 rows][128 B]
   float* sStat = reinterpret_cast<float*>(sdQ + 2 * TILE);   // QST x {-lse2[128], -dsum*scale[128]}
-  uint64_t* kv_full = reinterpret_cast<uint64_t*>(reinterpret_cast<uint8_t*>(sStat) + QST * STAT_BYTES);
+  uint64_t* kv_full = reinterpret_cast<uint64_t*>(reinterpret_cast<uint8_t*>(sStat) + QST * SB);
   uint64_t* kv_empty = kv_full + 1;        // the key tile's last MMAs retired: K / V may be replaced
   uint64_t* q_full = kv_empty + 1;         // [QST]
   uint64_t* q_empty = q_full + QST;        // [QST]
@@ -131,6 +142,8 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
   const int group = p.Hq / p.Hkv;
   const int col_k = (p.Hq + hk) * D, col_v = (p.Hq + p.Hkv + hk) * D;
   const bool dbg_cta = p.dbg != nullptr && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0;
+  // query tiles kb .. qend-1 of key tile kb
+  auto q_end = [&](int kb) { return MASKED ? p.q_hi[b * nq + kb] + 1 : nq; };
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmap_qkv);
@@ -170,12 +183,12 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
         tma_load_2d(sV, &tmap_qkv, kv_full, col_v, b * p.S + kb * BKV);
         for (int hh = 0; hh < group; ++hh) {
           const int h = hk * group + hh;
-          for (int qi = kb; qi < nq; ++qi) {
+          for (int qi = kb, qe = q_end(kb); qi < qe; ++qi) {
             mbar_wait(&q_empty[st], ph ^ 1);
-            mbar_arrive_expect_tx(&q_full[st], 2 * TILE + STAT_BYTES);
+            mbar_arrive_expect_tx(&q_full[st], 2 * TILE + SB);
             tma_load_2d(sQ + st * TILE, &tmap_qkv, &q_full[st], h * D, b * p.S + qi * BQ);
             tma_load_2d(sdO + st * TILE, &tmap_do, &q_full[st], h * D, b * p.S + qi * BQ);
-            bulk_load_1d(sStat + st * 256, p.stats + (((size_t)b * p.Hq + h) * nq + qi) * 256, STAT_BYTES, &q_full[st]);
+            bulk_load_1d(sStat + st * SF, p.stats + (((size_t)b * p.Hq + h) * nq + qi) * SF, SB, &q_full[st]);
             if (++st == QST) { st = 0; ph ^= 1; }
           }
         }
@@ -215,7 +228,8 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
         __syncwarp();
       };
       for (int w = 0, g = 0; w < nitems; ++w) {
-        const int iters = group * (nq - (w ? kb_second : kb_first));
+        const int kb = w ? kb_second : kb_first;
+        const int iters = group * (q_end(kb) - kb);
         mbar_wait(kv_full, w & 1);
         if (g > 0) mbar_wait(s_free, (g - 1) & 1);       // the previous key tile's last S^T has been read
         issue_s();
@@ -283,7 +297,7 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
       const int kb = w ? kb_second : kb_first;
       for (int hh = 0; hh < group; ++hh) {
         const int h = hk * group + hh;
-        for (int qi = kb; qi < nq; ++qi, ++it) {
+        for (int qi = kb, qe = q_end(kb); qi < qe; ++qi, ++it) {
           mbar_wait(mma_done, it & 1);
           tc_fence_after_sync();
           if (elected) tma_store_wait_read<0>();         // previous reduce finished reading the staging tile
@@ -332,10 +346,12 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
     int st = 0, ph = 0;
     for (int w = 0, it = 0; w < nitems; ++w) {
       const int kb = w ? kb_second : kb_first;
+      const int key = kb * BKV + row;                    // MASKED: this thread's key position and its valid bit
+      const bool key_valid = MASKED ? (p.vbits[(size_t)b * (p.S / 32) + key / 32] >> (key & 31)) & 1u : true;
       for (int hh = 0; hh < group; ++hh) {
-        for (int qi = kb; qi < nq; ++qi, ++it) {
+        for (int qi = kb, qe = q_end(kb); qi < qe; ++qi, ++it) {
           const bool diag = (qi == kb);
-          const uint32_t stat = smem_u32(sStat + st * 256 + part * NQ);
+          const uint32_t stat = smem_u32(sStat + st * SF + part * NQ);
           BWD_STAMP(0);
           mbar_wait(&q_full[st], ph);                    // the statistics of this query tile are in shared memory
           mbar_wait(s_full, it & 1);
@@ -350,7 +366,22 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
             __syncwarp();
             if (lane == 0) mbar_arrive(s_free);          // S^T(it+1) may now be computed into the same columns
             BWD_STAMP(2);
-            if (diag) {
+            if constexpr (MASKED) {
+              // queries qi*128 + part*NQ + i; the warp takes the causal code when none of its keys needs a masked element
+              const bool need = diag || !key_valid || key < p.lo_hi[b * nq + qi];
+              if (__any_sync(0xffffffffu, need)) {
+                const int rel = key - (qi * BQ + part * NQ);   // i == rel: the query is this key
+                const int* lo_s = reinterpret_cast<const int*>(sStat + st * SF + 256 + part * NQ);
+#pragma unroll
+                for (int i = 0; i < NQ; i += 4) {
+                  const int4 l4 = *reinterpret_cast<const int4*>(lo_s + i);
+                  const int lv[4] = {l4.x, l4.y, l4.z, l4.w};
+#pragma unroll
+                  for (int u = 0; u < 4; ++u)
+                    if (!(i + u >= rel && key >= lv[u] && (key_valid || i + u == rel))) sr[i + u] = 0xff800000u;
+                }
+              }
+            } else if (diag) {
 #pragma unroll
               for (int i = 0; i < NQ; ++i)
                 if (row > part * NQ + i) sr[i] = 0xff800000u;     // key after query: -inf -> P = 0
@@ -458,9 +489,12 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
 // Pre-pass: per (token, head) D = sum_d dO * O, stored together with the forward's log-sum-exp in the layout the main
 // kernel bulk-copies per query tile: stats[b, h, s/128, 0, s%128] = -lse * log2(e), stats[..., 1, ...] = -D * scale.
 // Eight lanes per (token, head) (16 bytes of dO and O each); the same threads zero the fp32 dQ accumulator row.
+// MASKED: a third row carries lo[s] (int32 bits).
+template <bool MASKED = false>
 __global__ void __launch_bounds__(256) attn_dsum_kernel(const __nv_bfloat16* __restrict__ dout, const __nv_bfloat16* __restrict__ out,
                                                         const float* __restrict__ lse, float* __restrict__ stats,
-                                                        float* __restrict__ dq_acc, int B, int S, int Hq, long long ld, float scale) {
+                                                        float* __restrict__ dq_acc, int B, int S, int Hq, long long ld, float scale,
+                                                        const int* __restrict__ lo = nullptr) {
   pdl_launch_dependents();
   pdl_wait();
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -484,9 +518,10 @@ __global__ void __launch_bounds__(256) attn_dsum_kernel(const __nv_bfloat16* __r
   z[1] = make_float4(0.f, 0.f, 0.f, 0.f);
   if (sub == 0) {
     const long long bb = t / S, ss = t % S;
-    float* dst = stats + (((bb * Hq + h) * (S / 128) + ss / 128) * 2) * 128 + (ss % 128);
+    float* dst = stats + (((bb * Hq + h) * (S / 128) + ss / 128) * (MASKED ? 3 : 2)) * 128 + (ss % 128);
     dst[0] = -lse[(bb * Hq + h) * S + ss] * 1.4426950408889634f;
     dst[128] = -s * scale;
+    if (MASKED) dst[256] = __int_as_float(lo[t]);
   }
 }
 
@@ -546,21 +581,19 @@ ODB_EXPORT int odb_attn_bwd_set_dbg(void* buf) {
   return 0;
 }
 
-// stats: fp32 scratch of 2 * B * Hq * S elements (per-query statistics, written by the pre-pass);
-// dq_acc: fp32 [T, Hq*64] scratch (zeroed by the pre-pass, accumulated with TMA reduce-add);
-// dq, dk, dv: bf16 outputs with row strides ld_dq / ld_dkv elements - e.g. the three column blocks of one packed
-// [T, (Hq+2*Hkv)*64] buffer.  With cos/sin (fp32 [S, 32] tables) dq and dk leave with the RoPE rotation undone.
-ODB_EXPORT int odb_attn_bwd(const void* qkv, const void* out, const void* dout, const void* lse, void* stats, void* dq_acc,
-                            void* dq, void* dk, void* dv, const void* cos_t, const void* sin_t, int B, int S, int Hq, int Hkv,
-                            long long ld_qkv, long long ld_out, long long ld_dq, long long ld_dkv, float softmax_scale,
-                            cudaStream_t st) {
+namespace {
+template <bool MASKED>
+int launch_attn_bwd(const void* qkv, const void* out, const void* dout, const void* lse, void* stats, void* dq_acc, void* dq,
+                    void* dk, void* dv, const void* cos_t, const void* sin_t, int B, int S, int Hq, int Hkv, long long ld_qkv,
+                    long long ld_out, long long ld_dq, long long ld_dkv, float softmax_scale, const int* lo,
+                    const uint32_t* vbits, const int* q_hi, const int* lo_hi, cudaStream_t st) {
   using namespace attn_bwd;
   if (S % BQ || Hq % Hkv || ld_qkv % 8 || ld_out % 8 || ld_dq % 8 || ld_dkv % 8) return -1;
   const long long T = (long long)B * S;
   {
     const long long threads = T * Hq * 8;
-    launch_pdl(attn_dsum_kernel, dim3((unsigned)((threads + 255) / 256)), dim3(256), 0, st, (const __nv_bfloat16*)dout,
-               (const __nv_bfloat16*)out, (const float*)lse, (float*)stats, (float*)dq_acc, B, S, Hq, ld_out, softmax_scale);
+    launch_pdl(attn_dsum_kernel<MASKED>, dim3((unsigned)((threads + 255) / 256)), dim3(256), 0, st, (const __nv_bfloat16*)dout,
+               (const __nv_bfloat16*)out, (const float*)lse, (float*)stats, (float*)dq_acc, B, S, Hq, ld_out, softmax_scale, lo);
   }
   CUtensorMap tq, tdo, tdq, tdk, tdv;
   int rc;
@@ -575,17 +608,29 @@ ODB_EXPORT int odb_attn_bwd(const void* qkv, const void* out, const void* dout, 
   p.scale_log2 = softmax_scale * 1.4426950408889634f;
   p.stats = (const float*)stats;
   p.dbg = g_bwd_dbg;
-  static int ews = 0;
-  if (!ews) {
-    const char* env = getenv("ODB_ATTN_BWD_SPLIT");      // element-wise threads per key row: 2 or 4
-    ews = (env && atoi(env) == 2) ? 2 : (env && atoi(env) == 4) ? 4 : DEFAULT_EWS;
-    cudaError_t e = cudaFuncSetAttribute(attn_bwd_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_bwd_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e != cudaSuccess) { ews = 0; return (int)e; }
-  }
+  p.vbits = vbits; p.q_hi = q_hi; p.lo_hi = lo_hi;
   dim3 grid((S / BKV + 1) / 2, Hkv, B);
-  if (ews == 2) launch_pdl(attn_bwd_kernel<2>, grid, dim3(Roles<2>::THREADS), SMEM_BYTES, st, tq, tdo, tdq, tdk, tdv, p);
-  else launch_pdl(attn_bwd_kernel<4>, grid, dim3(Roles<4>::THREADS), SMEM_BYTES, st, tq, tdo, tdq, tdk, tdv, p);
+  if constexpr (MASKED) {
+    // two threads per key row (the default split) only
+    static bool attr_set = false;
+    if (!attr_set) {
+      cudaError_t e = cudaFuncSetAttribute(attn_bwd_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MASKED_SMEM_BYTES);
+      if (e != cudaSuccess) return (int)e;
+      attr_set = true;
+    }
+    launch_pdl(attn_bwd_kernel<2, true>, grid, dim3(Roles<2>::THREADS), MASKED_SMEM_BYTES, st, tq, tdo, tdq, tdk, tdv, p);
+  } else {
+    static int ews = 0;
+    if (!ews) {
+      const char* env = getenv("ODB_ATTN_BWD_SPLIT");      // element-wise threads per key row: 2 or 4
+      ews = (env && atoi(env) == 2) ? 2 : (env && atoi(env) == 4) ? 4 : DEFAULT_EWS;
+      cudaError_t e = cudaFuncSetAttribute(attn_bwd_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
+      if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_bwd_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
+      if (e != cudaSuccess) { ews = 0; return (int)e; }
+    }
+    if (ews == 2) launch_pdl(attn_bwd_kernel<2>, grid, dim3(Roles<2>::THREADS), SMEM_BYTES, st, tq, tdo, tdq, tdk, tdv, p);
+    else launch_pdl(attn_bwd_kernel<4>, grid, dim3(Roles<4>::THREADS), SMEM_BYTES, st, tq, tdo, tdq, tdk, tdv, p);
+  }
   {
     const long long threads = T * (Hq + (cos_t ? Hkv : 0)) * 4;
     launch_pdl(attn_bwd_finish_kernel, dim3((unsigned)((threads + 255) / 256)), dim3(256), 0, st, (const float*)dq_acc,
@@ -593,4 +638,29 @@ ODB_EXPORT int odb_attn_bwd(const void* qkv, const void* out, const void* dout, 
   }
   cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? 0 : (int)e;
+}
+}  // namespace
+
+// stats: fp32 scratch of 2 * B * Hq * S elements (per-query statistics, written by the pre-pass);
+// dq_acc: fp32 [T, Hq*64] scratch (zeroed by the pre-pass, accumulated with TMA reduce-add);
+// dq, dk, dv: bf16 outputs with row strides ld_dq / ld_dkv elements - e.g. the three column blocks of one packed
+// [T, (Hq+2*Hkv)*64] buffer.  With cos/sin (fp32 [S, 32] tables) dq and dk leave with the RoPE rotation undone.
+ODB_EXPORT int odb_attn_bwd(const void* qkv, const void* out, const void* dout, const void* lse, void* stats, void* dq_acc,
+                            void* dq, void* dk, void* dv, const void* cos_t, const void* sin_t, int B, int S, int Hq, int Hkv,
+                            long long ld_qkv, long long ld_out, long long ld_dq, long long ld_dkv, float softmax_scale,
+                            cudaStream_t st) {
+  return launch_attn_bwd<false>(qkv, out, dout, lse, stats, dq_acc, dq, dk, dv, cos_t, sin_t, B, S, Hq, Hkv, ld_qkv, ld_out,
+                                ld_dq, ld_dkv, softmax_scale, nullptr, nullptr, nullptr, nullptr, st);
+}
+
+// Same with a mask description (lo, vbits, q_hi, lo_hi from odb_attn_mask_prep); stats then holds 3 * B * Hq * S elements.
+ODB_EXPORT int odb_attn_bwd_masked(const void* qkv, const void* out, const void* dout, const void* lse, void* stats, void* dq_acc,
+                                   void* dq, void* dk, void* dv, const void* cos_t, const void* sin_t, int B, int S, int Hq,
+                                   int Hkv, long long ld_qkv, long long ld_out, long long ld_dq, long long ld_dkv,
+                                   float softmax_scale, const void* lo, const void* vbits, const void* q_hi, const void* lo_hi,
+                                   cudaStream_t st) {
+  if (!lo || !vbits || !q_hi || !lo_hi) return -1;
+  return launch_attn_bwd<true>(qkv, out, dout, lse, stats, dq_acc, dq, dk, dv, cos_t, sin_t, B, S, Hq, Hkv, ld_qkv, ld_out, ld_dq,
+                               ld_dkv, softmax_scale, (const int*)lo, (const uint32_t*)vbits, (const int*)q_hi,
+                               (const int*)lo_hi, st);
 }

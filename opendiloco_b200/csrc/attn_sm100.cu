@@ -12,9 +12,15 @@
 //              64-127, row max exchanged through shared memory): tcgen05.ld S, online max/sum with exp2, causal mask
 //              on the diagonal tile, rescale O in TMEM (tcgen05.ld/st), write P (bf16) into the swizzled smem operand;
 //              epilogue: O / l -> bf16 -> swizzled staging tile -> TMA store
+//
+// MASKED instantiation (padding / per-document masks, described by odb_attn_mask_prep below): every role walks key tiles
+// kv_lo[b, qt] .. qt instead of 0 .. qt; a warp whose rows see only allowed keys in a tile takes the causal code, the
+// others apply allowed(s, t) = t == s || (lo[s] <= t < s && valid[t]) as -inf.  A row may meet fully masked tiles before
+// its first allowed key, so the online softmax keeps its reference at -inf without producing NaN there.
 #include "common.cuh"
 #include "sm100_ptx.cuh"
 #include "packed_math.cuh"
+#include <climits>
 
 using namespace odb;
 using namespace sm100;
@@ -38,10 +44,15 @@ struct Params {
   float scale_log2;        // softmax_scale * log2(e)
   float* lse;              // [B, Hq, S], natural log
   long long* dbg;          // optional timeline of CTA (0,0,0): [tile][16] clock64 stamps (nullptr = off)
+  // MASKED only (odb_attn_mask_prep outputs)
+  const int* lo;           // [B*S] first allowed key of every query
+  const uint32_t* vbits;   // [B, S/32] key-valid bits
+  const int* kv_lo;        // [B, S/128] first key tile a query tile visits
 };
 
 #define ATT_STAMP(slot) do { if (dbg_on) p.dbg[j * 16 + (slot)] = clock64(); } while (0)
 
+template <bool MASKED>
 __global__ void __launch_bounds__(THREADS, 2)
 attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_constant__ CUtensorMap tmap_out, Params p) {
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -109,17 +120,18 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
         tma_load_2d(sK + st * TILE_BYTES, &tmap_qkv, &k_full[st], col_k, b * p.S + j * BKV);
       };
       for (int w = 0, t0 = 0; w < nitems; ++w) {
-        const int nkv = qb[w] + 1;               // causal: key tiles 0..qblk
+        const int j0 = MASKED ? p.kv_lo[b * nq + qb[w]] : 0;
+        const int nkv = qb[w] + 1 - j0;          // causal: key tiles j0..qblk
         mbar_wait(q_empty, (w & 1) ^ 1);
         mbar_arrive_expect_tx(q_full, TILE_BYTES);
         tma_load_2d(sQ, &tmap_qkv, q_full, col_q, b * p.S + qb[w] * BQ);
-        load_k(0, t0);
+        load_k(j0, t0);
         for (int j = 0; j < nkv; ++j) {
           const int tg = t0 + j;
-          if (j + 1 < nkv) load_k(j + 1, tg + 1);
+          if (j + 1 < nkv) load_k(j0 + j + 1, tg + 1);
           mbar_wait(v_empty, (tg & 1) ^ 1);
           mbar_arrive_expect_tx(v_full, TILE_BYTES);
-          tma_load_2d(sV, &tmap_qkv, v_full, col_v, b * p.S + j * BKV);
+          tma_load_2d(sV, &tmap_qkv, v_full, col_v, b * p.S + (j0 + j) * BKV);
         }
         t0 += nkv;
       }
@@ -150,7 +162,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
       __syncwarp();
     };
     for (int w = 0, t0 = 0; w < nitems; ++w) {
-    const int nkv = qb[w] + 1;
+    const int nkv = qb[w] + 1 - (MASKED ? p.kv_lo[b * nq + qb[w]] : 0);
     const bool dbg_on = dbg_cta && w == 0;
     mbar_wait(q_full, w & 1);
     if (w > 0) mbar_wait(s_free, (t0 - 1) & 1);  // the previous query tile's last S has been read
@@ -191,9 +203,13 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
     const float c = p.scale_log2;
     const bool dbg_cta = p.dbg != nullptr && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && threadIdx.x == 64;
     for (int w = 0, t0 = 0; w < nitems; ++w) {
-    const int qblk = qb[w], nkv = qblk + 1;
+    const int qblk = qb[w];
+    const int j0 = MASKED ? p.kv_lo[b * nq + qblk] : 0;
+    const int nkv = qblk + 1 - j0;
     const int row0 = b * p.S + qblk * BQ;        // first token row of this query tile
     const bool dbg_on = dbg_cta && w == 0;
+    const int qpos = qblk * BQ + row;            // MASKED: this row's query position and its first allowed key
+    const int lo_q = MASKED ? p.lo[b * p.S + qpos] : 0;
     float m = -INFINITY, l = 0.f;                // l: this thread's half of the row sum
     for (int j = 0; j < nkv; ++j) {
       const int tg = t0 + j;
@@ -201,7 +217,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
       mbar_wait(s_full, tg & 1);
       tc_fence_after_sync();
       ATT_STAMP(1);
-      const bool diag = (j == qblk);
+      const bool diag = (j0 + j == qblk);
       uint32_t sr[64];
       tmem_ld_32x32b_x32(tS + lane_off + half * 64, *reinterpret_cast<uint32_t(*)[32]>(&sr[0]));
       tmem_ld_32x32b_x32(tS + lane_off + half * 64 + 32, *reinterpret_cast<uint32_t(*)[32]>(&sr[32]));
@@ -210,7 +226,21 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
       __syncwarp();
       if (lane == 0) mbar_arrive(s_free);        // S_j now lives in registers
       ATT_STAMP(2);
-      if (diag) {
+      if constexpr (MASKED) {
+        // keys kbase + i of this thread; the warp takes the causal code when none of its rows needs a masked element
+        const int kbase = (j0 + j) * BKV + half * 64;
+        const uint32_t* vw = p.vbits + (size_t)b * (p.S / 32) + kbase / 32;
+        const uint32_t w0 = vw[0], w1 = vw[1];
+        const bool need = kbase + 63 > qpos || lo_q > kbase || (w0 & w1) != 0xffffffffu;
+        if (__any_sync(0xffffffffu, need)) {
+          const int rel_hi = qpos - kbase, rel_lo = lo_q - kbase;
+#pragma unroll
+          for (int i = 0; i < 64; ++i) {
+            const uint32_t bit = ((i < 32 ? w0 : w1) >> (i & 31)) & 1u;
+            if (!(i <= rel_hi && i >= rel_lo && (bit || i == rel_hi))) sr[i] = 0xff800000u;
+          }
+        }
+      } else if (diag) {
 #pragma unroll
         for (int i = 0; i < 64; ++i)
           if (half * 64 + i > row) sr[i] = 0xff800000u;      // -inf
@@ -233,8 +263,13 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
       // until then probabilities may exceed 1 (<= 2^8), which fp32 sums and bf16 P represent without trouble, and O / l
       // need no correction.  Both threads of a row see the same mx, so they take the same decision.
       if ((mx - m) * c <= 8.f) mx = m;
-      const float alpha = fast_exp2((m - mx) * c);   // m = -inf on the first tile -> 0
-      const float mc = mx * c;
+      float alpha = fast_exp2((m - mx) * c);         // m = -inf on the first tile -> 0
+      float mc = mx * c;
+      if constexpr (MASKED) {
+        // every key of this row so far is masked: keep m = -inf, l = 0 and O = 0 (P is 0 up to the 2^-126 floor of the
+        // polynomial, which the first allowed key's alpha = 0 wipes out) instead of -inf - -inf = NaN
+        if (mx == -INFINITY) { alpha = 1.f; mc = 0.f; }
+      }
       // p = exp2(s*c - m*c) with packed fp32x2 arithmetic (FFMA2 / FADD2).  Of every four elements two go through the
       // MUFU (ex2.approx) and two through a Cody-Waite + degree-3 polynomial on the FMA pipe, so both pipes work in
       // parallel (16384 exponentials per tile would otherwise keep the 16-lane MUFU busy for 1024 cycles per SM).
@@ -321,11 +356,115 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
   if (warp == 1) tmem_dealloc(tmem_base, TMEM_COLS);
 }
 
+
+// Mask description for the MASKED kernels (one CTA per row b; see ops/kernels.py::attn_mask_prep for the reference):
+//   valid[t]  = mask[b, t] != 0                      docstart[s] = 1 + last p < s with ids[b, p] == eos (0 when eos < 0)
+//   lo[s]     = min(s, first t >= docstart[s] with valid[t])
+//   vbits[b, t/32] bit t%32 = valid[t]   kv_lo[b, qt] = min lo / 128   lo_hi[b, qt] = max lo   over query tile qt
+//   q_hi[b, kt] = max{qt : kv_lo[b, qt] <= kt}
+// Chunked scans: thread c owns positions [c*ch, (c+1)*ch); the chunk aggregates are scanned across the block.
+constexpr int PREP_THREADS = 256;
+
+template <bool MAX>
+__device__ int block_scan_incl(int v, int* sh) {           // inclusive max / min scan in thread order
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int u = __shfl_up_sync(0xffffffffu, v, o);
+    if (lane >= o) v = MAX ? max(v, u) : min(v, u);
+  }
+  if (lane == 31) sh[warp] = v;
+  __syncthreads();
+  if (warp == 0) {
+    int t = lane < PREP_THREADS / 32 ? sh[lane] : (MAX ? INT_MIN : INT_MAX);
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int u = __shfl_up_sync(0xffffffffu, t, o);
+      if (lane >= o) t = MAX ? max(t, u) : min(t, u);
+    }
+    if (lane < PREP_THREADS / 32) sh[lane] = t;
+  }
+  __syncthreads();
+  if (warp > 0) v = MAX ? max(v, sh[warp - 1]) : min(v, sh[warp - 1]);
+  __syncthreads();
+  return v;
+}
+
+__device__ __forceinline__ bool mask_valid(const uint8_t* mask, int esz, long long i) {
+  if (mask == nullptr) return true;
+  const uint8_t* e = mask + i * esz;
+  uint8_t any = 0;
+  for (int k = 0; k < esz; ++k) any |= e[k];
+  return any != 0;
+}
+
+__global__ void __launch_bounds__(PREP_THREADS) attn_mask_prep_kernel(const long long* __restrict__ ids,
+                                                                      const uint8_t* __restrict__ mask, int esz, int S,
+                                                                      long long eos, int* __restrict__ lo,
+                                                                      uint32_t* __restrict__ vbits, int* __restrict__ kv_lo,
+                                                                      int* __restrict__ q_hi, int* __restrict__ lo_hi) {
+  extern __shared__ int nv[];                                // [S] first valid position >= p (S when none)
+  __shared__ int sh[32], agg[PREP_THREADS];
+  int* t_min = nv + S;                                       // [nq] per query tile: min lo, max lo
+  int* t_max = t_min + (S + 127) / 128;
+  pdl_launch_dependents();
+  pdl_wait();
+  const int b = blockIdx.x, tid = threadIdx.x, nq = (S + 127) / 128, nw = (S + 31) / 32;
+  const long long row = (long long)b * S;
+  const int ch = (S + PREP_THREADS - 1) / PREP_THREADS;
+  for (int q = tid; q < nq; q += PREP_THREADS) { t_min[q] = INT_MAX; t_max[q] = INT_MIN; }
+  for (int w = tid; w < nw; w += PREP_THREADS) {
+    uint32_t bits = 0;
+    for (int k = 0; k < 32 && w * 32 + k < S; ++k) bits |= (uint32_t)mask_valid(mask, esz, row + w * 32 + k) << k;
+    vbits[(long long)b * nw + w] = bits;
+  }
+  {  // suffix min of valid positions: thread tid owns chunk PREP_THREADS-1-tid, so a prefix scan over threads is a suffix scan
+    const int c = PREP_THREADS - 1 - tid, p0 = min(S, c * ch), p1 = min(S, p0 + ch);
+    int first = S;
+    for (int p = p1 - 1; p >= p0; --p) if (mask_valid(mask, esz, row + p)) first = p;
+    agg[tid] = block_scan_incl<false>(first, sh);
+    __syncthreads();
+    int cur = tid > 0 ? agg[tid - 1] : S;
+    for (int p = p1 - 1; p >= p0; --p) {
+      if (mask_valid(mask, esz, row + p)) cur = p;
+      nv[p] = cur;
+    }
+  }
+  __syncthreads();
+  {  // prefix max of (last EOS + 1), then lo
+    const int p0 = min(S, tid * ch), p1 = min(S, p0 + ch);
+    int ds = 0;
+    if (eos >= 0)
+      for (int p = p0; p < p1; ++p) if (ids[row + p] == eos) ds = p + 1;
+    agg[tid] = block_scan_incl<true>(ds, sh);
+    __syncthreads();
+    ds = tid > 0 ? agg[tid - 1] : 0;
+    for (int p = p0; p < p1; ++p) {
+      const int l = min(p, nv[ds]);
+      lo[row + p] = l;
+      atomicMin(&t_min[p / 128], l);
+      atomicMax(&t_max[p / 128], l);
+      if (eos >= 0 && ids[row + p] == eos) ds = p + 1;
+    }
+  }
+  __syncthreads();
+  for (int q = tid; q < nq; q += PREP_THREADS) {
+    kv_lo[(long long)b * nq + q] = t_min[q] / 128;
+    lo_hi[(long long)b * nq + q] = t_max[q];
+  }
+  for (int kt = tid; kt < nq; kt += PREP_THREADS) {
+    int hi = kt;                                             // kv_lo[kt] <= kt always
+    for (int q = nq - 1; q > kt; --q)
+      if (t_min[q] / 128 <= kt) { hi = q; break; }
+    q_hi[(long long)b * nq + kt] = hi;
+  }
+}
 }  // namespace attn
 
-// qkv: [B*S, (Hq+2*Hkv)*64] bf16 (row stride ld_qkv elements); out: [B*S, Hq*64] bf16; lse: [B, Hq, S] fp32
-ODB_EXPORT int odb_attn_fwd(const void* qkv, void* out, void* lse, int B, int S, int Hq, int Hkv, long long ld_qkv,
-                            long long ld_out, float softmax_scale, void* dbg, cudaStream_t st) {
+namespace {
+template <bool MASKED>
+int launch_attn_fwd(const void* qkv, void* out, void* lse, int B, int S, int Hq, int Hkv, long long ld_qkv, long long ld_out,
+                    float softmax_scale, void* dbg, const int* lo, const uint32_t* vbits, const int* kv_lo, cudaStream_t st) {
   using namespace attn;
   if (S % BQ || Hq % Hkv || ld_qkv % 8 || ld_out % 8) return -1;
   CUtensorMap tq, to;
@@ -338,14 +477,50 @@ ODB_EXPORT int odb_attn_fwd(const void* qkv, void* out, void* lse, int B, int S,
   p.scale_log2 = softmax_scale * 1.4426950408889634f;
   p.lse = (float*)lse;
   p.dbg = (long long*)dbg;
+  p.lo = lo; p.vbits = vbits; p.kv_lo = kv_lo;
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(attn_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
+    cudaError_t e = cudaFuncSetAttribute(attn_fwd_kernel<MASKED>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
     if (e != cudaSuccess) return (int)e;
     attr_set = true;
   }
   dim3 grid((S / BQ + 1) / 2, Hq, B);
-  launch_pdl(attn_fwd_kernel, grid, dim3(THREADS), SMEM_BYTES, st, tq, to, p);
+  launch_pdl(attn_fwd_kernel<MASKED>, grid, dim3(THREADS), SMEM_BYTES, st, tq, to, p);
+  cudaError_t e = cudaGetLastError();
+  return e == cudaSuccess ? 0 : (int)e;
+}
+}  // namespace
+
+// qkv: [B*S, (Hq+2*Hkv)*64] bf16 (row stride ld_qkv elements); out: [B*S, Hq*64] bf16; lse: [B, Hq, S] fp32
+ODB_EXPORT int odb_attn_fwd(const void* qkv, void* out, void* lse, int B, int S, int Hq, int Hkv, long long ld_qkv,
+                            long long ld_out, float softmax_scale, void* dbg, cudaStream_t st) {
+  return launch_attn_fwd<false>(qkv, out, lse, B, S, Hq, Hkv, ld_qkv, ld_out, softmax_scale, dbg, nullptr, nullptr, nullptr, st);
+}
+
+// Same with a mask description (lo, vbits, kv_lo from odb_attn_mask_prep).
+ODB_EXPORT int odb_attn_fwd_masked(const void* qkv, void* out, void* lse, int B, int S, int Hq, int Hkv, long long ld_qkv,
+                                   long long ld_out, float softmax_scale, const void* lo, const void* vbits, const void* kv_lo,
+                                   cudaStream_t st) {
+  if (!lo || !vbits || !kv_lo) return -1;
+  return launch_attn_fwd<true>(qkv, out, lse, B, S, Hq, Hkv, ld_qkv, ld_out, softmax_scale, nullptr, (const int*)lo,
+                               (const uint32_t*)vbits, (const int*)kv_lo, st);
+}
+
+// ids: int64 [B, S]; mask: optional [B, S] of any integer / bool type (mask_elem_bytes per element); eos < 0: no document
+// masking.  Outputs (int32): lo [B*S], vbits [B, ceil(S/32)], kv_lo / q_hi / lo_hi [B, ceil(S/128)].
+ODB_EXPORT int odb_attn_mask_prep(const void* ids, const void* mask, int mask_elem_bytes, int B, int S, long long eos, void* lo,
+                                  void* vbits, void* kv_lo, void* q_hi, void* lo_hi, cudaStream_t st) {
+  using namespace attn;
+  if (B <= 0 || S <= 0 || (mask && mask_elem_bytes <= 0)) return -1;
+  const size_t smem = ((size_t)S + 2 * ((S + 127) / 128)) * sizeof(int);
+  static size_t smem_set = 48 * 1024;
+  if (smem > smem_set) {
+    cudaError_t e = cudaFuncSetAttribute(attn_mask_prep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return (int)e;
+    smem_set = smem;
+  }
+  launch_pdl(attn_mask_prep_kernel, dim3(B), dim3(PREP_THREADS), smem, st, (const long long*)ids, (const uint8_t*)mask,
+             mask_elem_bytes, S, eos, (int*)lo, (uint32_t*)vbits, (int*)kv_lo, (int*)q_hi, (int*)lo_hi);
   cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? 0 : (int)e;
 }

@@ -88,6 +88,7 @@ class _Workspace:
         self._dev, self._dt, self._V = device, dtype, cfg.vocab_size
         self._logits = None          # reference path only (CPU / fp32 / fp16): bf16 kernels never materialise logits
         self._lce = None             # fused LCE buffers, allocated on first use
+        self._mask = None            # padding mask (int32 [B, S]) + its attention description, allocated on first use
         self.loss_sum = torch.zeros(1, dtype=f32, device=device)
         self.gscale = torch.ones(1, dtype=f32, device=device)
         self.n_valid = torch.ones(1, dtype=f32, device=device)
@@ -99,6 +100,12 @@ class _Workspace:
         if self._logits is None:
             self._logits = torch.empty(self.lce_rows, self._V, dtype=self._dt, device=self._dev)
         return self._logits
+
+    def mask_buffers(self) -> tuple[torch.Tensor, A.MaskDesc]:
+        """(static device copy of the padding mask, attention mask description) of this shape."""
+        if self._mask is None:
+            self._mask = (torch.empty(self.B, self.S, dtype=torch.int32, device=self._dev), A.MaskDesc.empty(self.B, self.S, self._dev))
+        return self._mask
 
     def lce_buffers(self, planes: int, h: int):
         """(shift [T], rowscale [T], partials [2*planes, C], e [C, V] bf16, xs [C, h] bf16) of the fused LCE."""
@@ -143,7 +150,27 @@ class LlamaEngine:
             for hook in list(mod._forward_hooks.values()):
                 hook(mod, (), out)
 
-    def forward_hidden(self, ws: _Workspace, ids: torch.Tensor, attention_mask: torch.Tensor | None = None) -> torch.Tensor:
+    def describe_mask(self, ws: _Workspace, ids: torch.Tensor, attention_mask: torch.Tensor | None,
+                      document_mask: bool = False) -> A.MaskDesc | None:
+        """Attention mask description of one micro-batch in the workspace's static buffers (None: plain causal).
+        ``attention_mask`` [B, S] as returned by ``_normalize_mask``; ``document_mask`` also keeps every query inside its
+        document (documents end with ``config.eos_token_id``)."""
+        if attention_mask is None and not document_mask:
+            return None
+        if attention_mask is not None and tuple(attention_mask.shape) != (ws.B, ws.S):
+            raise ValueError(f"attention_mask has shape {tuple(attention_mask.shape)}, expected {(ws.B, ws.S)}")
+        eos = -1
+        if document_mask:
+            if self.cfg.eos_token_id is None or self.cfg.eos_token_id < 0:
+                raise ValueError("document_mask needs config.eos_token_id")
+            eos = int(self.cfg.eos_token_id)
+        ws.ids.copy_(ids.reshape(-1), non_blocking=True)
+        mbuf, desc = ws.mask_buffers()
+        if attention_mask is not None:
+            mbuf.copy_(attention_mask, non_blocking=True)
+        return desc.build(ws.ids.view(ws.B, ws.S), mbuf if attention_mask is not None else None, eos)
+
+    def forward_hidden(self, ws: _Workspace, ids: torch.Tensor, mask: A.MaskDesc | None = None) -> torch.Tensor:
         cfg, ar = self.cfg, self.arena
         B, S, L = ws.B, ws.S, cfg.num_hidden_layers
         Hq, Hkv, D = cfg.num_attention_heads, cfg.num_key_value_heads, cfg.head_dim
@@ -162,10 +189,7 @@ class LlamaEngine:
             else:
                 G.mm_nt(ws.xn1[l], ar.qkv_w(l), out=ws.qkv[l])
                 K.rope_(ws.qkv[l], ws.cos, ws.sin, S, Hq + Hkv, D)
-            if attention_mask is None:
-                ws.att[l], ws.aux[l] = A.attention_fwd(ws.qkv[l], B, S, Hq, Hkv, D)
-            else:
-                ws.att[l], ws.aux[l] = _masked_attention_fwd(ws.qkv[l], attention_mask, B, S, Hq, Hkv, D)
+            ws.att[l], ws.aux[l] = A.attention_fwd(ws.qkv[l], B, S, Hq, Hkv, D, mask=mask)
             G.mm_nt(ws.att[l], ar.w(p + "self_attn.o_proj.weight"), out=ws.proj)
             if self.collect_act_norms:
                 self.act_norms[f"activation/{p}self_attn"] = ws.proj.float().norm(p=2)
@@ -285,7 +309,7 @@ class LlamaEngine:
         return G.mm_nt(ws.xnf, self.arena.w("lm_head.weight"))
 
     # --------------------------------------------------------------------------------------------- backward
-    def backward(self, ws: _Workspace, attention_mask: torch.Tensor | None = None) -> None:
+    def backward(self, ws: _Workspace, mask: A.MaskDesc | None = None) -> None:
         """Back-propagate ws.dxnf (gradient w.r.t. the final-norm output) through the stack, accumulating into arena.grad."""
         cfg, ar = self.cfg, self.arena
         B, S, L = ws.B, ws.S, cfg.num_hidden_layers
@@ -308,14 +332,9 @@ class LlamaEngine:
             # ---- attention block (ws.dx is now the gradient of xm = xa + o(att))
             G.mm_tn_acc(ws.dx, ws.att[l], ar.g(p + "self_attn.o_proj.weight"))
             G.mm_nn(ws.dx, ar.w(p + "self_attn.o_proj.weight"), out=ws.datt)
-            parts_ok = (attention_mask is None and cfg.q_dim % 64 == 0 and cfg.kv_dim % 64 == 0
-                        and TC.nn_usable(ws.datt, ar.qkv_w(l)))
-            if attention_mask is None:
-                res = A.attention_bwd(ws.datt, ws.qkv[l], ws.att[l], ws.aux[l], ws.dqkv, B, S, Hq, Hkv, D, want_parts=parts_ok,
-                                      rope=(ws.cos, ws.sin))
-            else:
-                _masked_attention_bwd(ws.datt, ws.aux[l], ws.dqkv, B, S, Hq, Hkv, D)
-                res = ws.dqkv
+            parts_ok = cfg.q_dim % 64 == 0 and cfg.kv_dim % 64 == 0 and TC.nn_usable(ws.datt, ar.qkv_w(l))
+            res = A.attention_bwd(ws.datt, ws.qkv[l], ws.att[l], ws.aux[l], ws.dqkv, B, S, Hq, Hkv, D, want_parts=parts_ok,
+                                  rope=(ws.cos, ws.sin), mask=mask)
             if isinstance(res, tuple):
                 # un-packed gradients (cuDNN): rotate dq/dk in place, three wgrads into the row blocks of the fused
                 # QKV gradient, and ONE dgrad GEMM whose A operand is read from the three tensors
@@ -331,7 +350,7 @@ class LlamaEngine:
                     G.mm_tn_acc(dv, ws.xn1[l], gq[cfg.q_dim + cfg.kv_dim:])
                 TC.linear_nn_a3(dq, dk, dv, ar.qkv_w(l), ws.dn)
             else:
-                if attention_mask is not None or not A.bwd_applies_rope(ws.aux[l]):
+                if not A.bwd_applies_rope(ws.aux[l]):
                     K.rope_(ws.dqkv, ws.cos, ws.sin, S, Hq + Hkv, D, backward=True)
                 G.mm_tn_acc(ws.dqkv, ws.xn1[l], ar.qkv_g(l))
                 G.mm_nn(ws.dqkv, ar.qkv_w(l), out=ws.dn)
@@ -343,14 +362,15 @@ class LlamaEngine:
 
     # --------------------------------------------------------------------------------------------- fused entry
     def forward_backward(self, ids: torch.Tensor, labels: torch.Tensor, loss_scale: float = 1.0,
-                         attention_mask: torch.Tensor | None = None) -> torch.Tensor:
+                         attention_mask: torch.Tensor | None = None, document_mask: bool = False) -> torch.Tensor:
         """One micro-batch: forward, loss, backward; gradients (scaled by loss_scale) are ADDED to arena.grad.
-        Returns the mean token loss as a device scalar (no host sync)."""
+        Returns the mean token loss as a device scalar (no host sync).  ``attention_mask``: None or a [B, S] mask that is
+        not all ones (``_normalize_mask``; no host sync here, so the call can be captured into a CUDA graph)."""
         B, S = ids.shape
         ws = self.workspace(B, S)
-        mask = _normalize_mask(attention_mask)
         ar = self.arena
         with torch.no_grad():
+            mask = self.describe_mask(ws, ids, attention_mask, document_mask)
             ar.materialize_shadow()            # FULL_SHARD: all-gather the compute weights (no-op otherwise)
             self.forward_hidden(ws, ids, mask)
             loss = self.head_loss(ws, labels, loss_scale, with_grad=True, direct=True)
@@ -363,17 +383,21 @@ class LlamaEngine:
 
 
     # --------------------------------------------------------------------------------------------- CUDA-graph replay
-    def forward_backward_graphed(self, ids: torch.Tensor, labels: torch.Tensor, loss_scale: float) -> torch.Tensor:
-        """``forward_backward`` with the ~250 launches of a micro-batch captured ONCE per (B, S, loss_scale) into a CUDA
-        graph and replayed afterwards (every buffer of the micro-step is static: workspace, arena, TMA descriptors are
-        baked kernel parameters).  Inputs are copied into the graph's static id / label buffers; the returned loss is the
-        graph's static output (consume it before the next replay).  Falls back to the eager path while hooks /
-        activation-norm collection are active (they run Python between kernels)."""
+    def forward_backward_graphed(self, ids: torch.Tensor, labels: torch.Tensor, loss_scale: float,
+                                 attention_mask: torch.Tensor | None = None, document_mask: bool = False) -> torch.Tensor:
+        """``forward_backward`` with the ~250 launches of a micro-batch captured ONCE per (B, S, loss_scale, masked,
+        document_mask) into a CUDA graph and replayed afterwards (every buffer of the micro-step is static: workspace,
+        arena, TMA descriptors are baked kernel parameters).  Inputs (ids, labels, the padding mask) are copied into the
+        graph's static buffers and the mask description is computed inside the graph; the returned loss is the graph's
+        static output (consume it before the next replay).  ``attention_mask`` must be normalised (``_normalize_mask``).
+        Falls back to the eager path while hooks / activation-norm collection are active (they run Python between
+        kernels)."""
         B, S = ids.shape
         hooked = any(m._forward_hooks for m in self.module_hooks.values())
         if self.collect_act_norms or hooked or not ids.is_cuda:
-            return self.forward_backward(ids, labels, loss_scale)
-        key = (B, S, float(loss_scale), labels is ids)
+            return self.forward_backward(ids, labels, loss_scale, attention_mask, document_mask)
+        masked = attention_mask is not None
+        key = (B, S, float(loss_scale), labels is ids, masked, bool(document_mask))
         st = self._graphs.get(key)
         if st is not None and st.get("version") != self.arena.version:
             st = None                     # an arena buffer was re-homed (symmetric-memory windows): captured pointers are stale
@@ -383,12 +407,15 @@ class LlamaEngine:
         if st["graph"] is None:
             st["calls"] += 1
             if st["calls"] <= 2:          # warm-up: allocations, cudaFuncSetAttribute, library handles
-                return self.forward_backward(ids, labels, loss_scale)
+                return self.forward_backward(ids, labels, loss_scale, attention_mask, document_mask)
             g_ids = torch.empty_like(ids)
             g_lab = g_ids if labels is ids else torch.empty_like(labels)
+            g_mask = torch.empty(B, S, dtype=torch.int32, device=ids.device) if masked else None
             g_ids.copy_(ids)
             if g_lab is not g_ids:
                 g_lab.copy_(labels)
+            if masked:
+                g_mask.copy_(attention_mask)
             ws = self.workspace(B, S)
             for l in range(self.cfg.num_hidden_layers):
                 ws.att[l] = ws.aux[l] = None
@@ -397,14 +424,16 @@ class LlamaEngine:
             n0 = _lib.launch_count()
             # thread_local: the NCCL watchdog / data-loader threads keep making CUDA calls of their own during the capture
             with torch.cuda.graph(graph, capture_error_mode="thread_local"):
-                loss = self.forward_backward(g_ids, g_lab, loss_scale)
+                loss = self.forward_backward(g_ids, g_lab, loss_scale, g_mask, document_mask)
             # kernels of ours recorded in the graph: every replay launches them again (bench.py's gpu_launches book-keeping)
-            st.update(graph=graph, ids=g_ids, labels=g_lab, loss=loss, kernels=_lib.launch_count() - n0)
+            st.update(graph=graph, ids=g_ids, labels=g_lab, mask=g_mask, loss=loss, kernels=_lib.launch_count() - n0)
             graph.replay()
             return st["loss"]
         st["ids"].copy_(ids, non_blocking=True)
         if st["labels"] is not st["ids"]:
             st["labels"].copy_(labels, non_blocking=True)
+        if masked:
+            st["mask"].copy_(attention_mask, non_blocking=True)
         st["graph"].replay()
         _lib.count_launch(st["kernels"])
         return st["loss"]
@@ -421,36 +450,14 @@ class _NormOnly:
 
 
 def _normalize_mask(attention_mask: torch.Tensor | None) -> torch.Tensor | None:
-    """None when the mask is absent or all ones (pure causal fast path)."""
+    """None when the mask is absent or all ones (pure causal fast path); otherwise the [B, S] mask as bool."""
     if attention_mask is None:
         return None
+    if attention_mask.dim() != 2:
+        raise ValueError(f"attention_mask must be 2-D [batch, seq], got shape {tuple(attention_mask.shape)}")
     if bool(attention_mask.all()):
         return None
     return attention_mask.bool()
-
-
-def _masked_attention_fwd(qkv, mask, B, S, Hq, Hkv, D):
-    """Padding-mask path (real text with pad tokens): library SDPA with an explicit mask, differentiated by autograd."""
-    q, k, v = A.split_qkv(qkv, B, S, Hq, Hkv, D)
-    leaves = [t.detach().transpose(1, 2).requires_grad_(True) for t in (q, k, v)]
-    causal = torch.ones(S, S, dtype=torch.bool, device=qkv.device).tril()
-    full = causal[None, None] & mask[:, None, None, :].to(qkv.device)
-    # keep fully-masked rows finite (pad queries): let them see themselves
-    full = full | torch.eye(S, dtype=torch.bool, device=qkv.device)[None, None]
-    with torch.enable_grad():
-        o = torch.nn.functional.scaled_dot_product_attention(leaves[0], leaves[1], leaves[2], attn_mask=full,
-                                                             enable_gqa=(Hq != Hkv))
-        out = o.transpose(1, 2).reshape(B * S, Hq * D)
-    return out.detach(), (out, leaves)
-
-
-def _masked_attention_bwd(dout, aux, dqkv, B, S, Hq, Hkv, D):
-    out, leaves = aux
-    gq, gk, gv = torch.autograd.grad(out, leaves, dout)
-    dq, dk, dv = A.split_qkv(dqkv, B, S, Hq, Hkv, D)
-    dq.copy_(gq.transpose(1, 2))
-    dk.copy_(gk.transpose(1, 2))
-    dv.copy_(gv.transpose(1, 2))
 
 
 # ======================================================================================================= nn.Module facade
@@ -470,10 +477,11 @@ class _EngineLoss(torch.autograd.Function):
     """Single autograd node bridging loss.backward() to the engine's hand-written backward."""
 
     @staticmethod
-    def forward(ctx, anchor: torch.Tensor, model: "LlamaForCausalLM", ids, labels, mask):
+    def forward(ctx, anchor: torch.Tensor, model: "LlamaForCausalLM", ids, labels, mask, document_mask):
         eng = model.engine
         B, S = ids.shape
         ws = eng.workspace(B, S)
+        mask = eng.describe_mask(ws, ids, mask, document_mask)
         eng.arena.materialize_shadow()
         eng.forward_hidden(ws, ids, mask)
         loss = eng.head_loss(ws, labels, 1.0, with_grad=True, direct=False)
@@ -491,7 +499,7 @@ class _EngineLoss(torch.autograd.Function):
             eng.arena.materialize_shadow()
             eng.backward(ws, ctx.mask)
             eng.arena.release_shadow()
-        return None, None, None, None, None
+        return None, None, None, None, None, None
 
 
 class LlamaForCausalLM(nn.Module):
@@ -579,7 +587,10 @@ class LlamaForCausalLM(nn.Module):
 
     # ------------------------------------------------------------------ forward
     def forward(self, input_ids: torch.Tensor, attention_mask: torch.Tensor | None = None,
-                labels: torch.Tensor | None = None, return_logits: bool = False, **_unused) -> CausalLMOutput:
+                labels: torch.Tensor | None = None, return_logits: bool = False, document_mask: bool = False,
+                **_unused) -> CausalLMOutput:
+        """``attention_mask`` [B, S]: 0 marks padding keys.  ``document_mask``: attention also stays inside the documents of
+        a packed row, each ending with ``config.eos_token_id`` (labels are not changed)."""
         eng = self.engine
         if input_ids.device != self.arena.device:
             input_ids = input_ids.to(self.arena.device, non_blocking=True)
@@ -588,25 +599,27 @@ class LlamaForCausalLM(nn.Module):
         mask = _normalize_mask(attention_mask)
         B, S = input_ids.shape
         if labels is not None and torch.is_grad_enabled() and self.training:
-            loss = _EngineLoss.apply(self.lm_head.weight, self, input_ids, labels, mask)
+            loss = _EngineLoss.apply(self.lm_head.weight, self, input_ids, labels, mask, document_mask)
             return CausalLMOutput(loss=loss)
         with torch.no_grad():
             ws = eng.workspace(B, S)
+            desc = eng.describe_mask(ws, input_ids, mask, document_mask)
             self.arena.materialize_shadow()
-            eng.forward_hidden(ws, input_ids, mask)
+            eng.forward_hidden(ws, input_ids, desc)
             loss = eng.head_loss(ws, labels, 1.0, with_grad=False, direct=False).clone() if labels is not None else None
             logits = eng.logits(ws).view(B, S, -1) if (return_logits or labels is None) else None
             self.arena.release_shadow()
         return CausalLMOutput(loss=loss, logits=logits)
 
     def forward_backward(self, input_ids: torch.Tensor, labels: torch.Tensor, loss_scale: float = 1.0,
-                         attention_mask: torch.Tensor | None = None) -> torch.Tensor:
+                         attention_mask: torch.Tensor | None = None, document_mask: bool = False) -> torch.Tensor:
         """Native fast path: one micro-batch forward+backward, grads += loss_scale * dL/dw. Returns the device loss.
-        With ODB_CUDA_GRAPH=1 (and no padding mask) the micro-step is replayed from a CUDA graph."""
-        if (_use_graph() and attention_mask is None and input_ids.is_cuda and self.arena.compute_dtype == torch.bfloat16
-                and not self.arena.param_sharded):
-            return self.engine.forward_backward_graphed(input_ids, labels, loss_scale)
-        return self.engine.forward_backward(input_ids, labels, loss_scale, attention_mask)
+        With ODB_CUDA_GRAPH=1 the micro-step is replayed from a CUDA graph (masked or not).  ``attention_mask`` /
+        ``document_mask`` as in ``forward``."""
+        mask = _normalize_mask(attention_mask)
+        if _use_graph() and input_ids.is_cuda and self.arena.compute_dtype == torch.bfloat16 and not self.arena.param_sharded:
+            return self.engine.forward_backward_graphed(input_ids, labels, loss_scale, mask, document_mask)
+        return self.engine.forward_backward(input_ids, labels, loss_scale, mask, document_mask)
 
     # ------------------------------------------------------------------ state dict / checkpoints
     def load_state_dict(self, state_dict, strict: bool = True, assign: bool = False):

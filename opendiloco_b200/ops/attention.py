@@ -10,6 +10,10 @@ Back-ends:
   * ``flash``  - flash-attn 2.8 library kernels (sm_80 mma.sync code: 266/196 TF/s on B200), ODB_ATTN_LIB=flash
   * ``math``   - fp32 PyTorch reference (CPU, tests)
 The reference framework itself calls a library here (torch SDPA / flash-attn: train_fsdp.py:107,173).
+
+Padding and per-document masks travel as a ``MaskDesc`` (``kernels.attn_mask_prep``): the ``tc`` back-end runs the
+MASKED instantiations of its kernels on it; every other case expands it with ``dense_mask`` - the math reference on the
+CPU, torch SDPA with that boolean mask on CUDA.
 """
 from __future__ import annotations
 
@@ -19,8 +23,10 @@ import os
 import torch
 
 import ctypes
+from dataclasses import dataclass
 
 from .. import _lib
+from . import kernels as K
 
 _FLASH = None
 # Back-end of the bf16 CUDA path: "tc" = our tcgen05 kernels (csrc/attn_sm100.cu, attn_bwd_sm100.cu; head_dim 64,
@@ -42,30 +48,71 @@ _lib.register_optional("odb_attn_fwd", [ctypes.c_void_p, ctypes.c_void_p, ctypes
 
 
 _lib.register_optional("odb_attn_bwd", [ctypes.c_void_p] * 11 + [ctypes.c_int] * 4 + [ctypes.c_longlong] * 4 + [ctypes.c_float, ctypes.c_void_p])
+_lib.register_optional("odb_attn_fwd_masked", [ctypes.c_void_p] * 3 + [ctypes.c_int] * 4 + [ctypes.c_longlong] * 2
+                       + [ctypes.c_float] + [ctypes.c_void_p] * 4)
+_lib.register_optional("odb_attn_bwd_masked", [ctypes.c_void_p] * 11 + [ctypes.c_int] * 4 + [ctypes.c_longlong] * 4
+                       + [ctypes.c_float] + [ctypes.c_void_p] * 5)
 _SCRATCH: dict = {}
 
 
-def _bwd_scratch(dev, T: int, Hq: int, D: int):
+@dataclass
+class MaskDesc:
+    """Per-batch description of a padding and/or per-document causal mask (int32 tensors written by
+    ``kernels.attn_mask_prep``, which documents the semantics): lo [B*S], vbits [B, ceil(S/32)], kv_lo / q_hi / lo_hi
+    [B, ceil(S/128)]."""
+    lo: torch.Tensor
+    vbits: torch.Tensor
+    kv_lo: torch.Tensor
+    q_hi: torch.Tensor
+    lo_hi: torch.Tensor
+
+    @classmethod
+    def empty(cls, B: int, S: int, device) -> "MaskDesc":
+        i32 = dict(dtype=torch.int32, device=device)
+        nq = (S + 127) // 128
+        return cls(torch.empty(B * S, **i32), torch.empty(B, (S + 31) // 32, **i32), torch.empty(B, nq, **i32),
+                   torch.empty(B, nq, **i32), torch.empty(B, nq, **i32))
+
+    def build(self, ids: torch.Tensor, mask: torch.Tensor | None, eos: int) -> "MaskDesc":
+        """Describe ``mask`` ([B, S], nonzero = real token; None = all ones) and, with ``eos >= 0``, the documents of ``ids``."""
+        K.attn_mask_prep(ids, mask, eos, self.lo, self.vbits, self.kv_lo, self.q_hi, self.lo_hi)
+        return self
+
+
+def dense_mask(desc: MaskDesc, B: int, S: int) -> torch.Tensor:
+    """Boolean [B, 1, S, S] mask (True = attend) of a description: ``t == s or (lo[s] <= t < s and valid[t])``."""
+    dev = desc.lo.device
+    t = torch.arange(S, device=dev)
+    valid = ((desc.vbits.long()[:, t // 32] >> (t % 32)) & 1).bool()
+    lo = desc.lo.view(B, S).long()
+    allowed = (lo[:, :, None] <= t) & (t < t[:, None]) & valid[:, None, :]
+    return (allowed | torch.eye(S, dtype=torch.bool, device=dev))[:, None]
+
+
+def _bwd_scratch(dev, T: int, Hq: int, D: int, masked: bool = False):
     """fp32 dQ accumulator + per-query statistics of the backward kernel (reused across layers / steps: every call
-    rewrites them completely before reading)."""
-    key = (dev, T, Hq, D)
+    rewrites them completely before reading).  The masked kernel keeps a third statistics row."""
+    key = (dev, T, Hq, D) if not masked else (dev, T, Hq, D, True)
     sc = _SCRATCH.get(key)
     if sc is None:
-        sc = (torch.empty(T, Hq * D, dtype=torch.float32, device=dev), torch.empty(2 * T * Hq, dtype=torch.float32, device=dev))
+        sc = (torch.empty(T, Hq * D, dtype=torch.float32, device=dev),
+              torch.empty((3 if masked else 2) * T * Hq, dtype=torch.float32, device=dev))
         _SCRATCH[key] = sc
     return sc
 
 
 def tc_attention_bwd(dout: torch.Tensor, qkv: torch.Tensor, out: torch.Tensor, lse: torch.Tensor, B: int, S: int, Hq: int, Hkv: int,
-                     D: int = 64, dqkv: torch.Tensor | None = None, cos: torch.Tensor | None = None, sin: torch.Tensor | None = None):
+                     D: int = 64, dqkv: torch.Tensor | None = None, cos: torch.Tensor | None = None, sin: torch.Tensor | None = None,
+                     mask: MaskDesc | None = None):
     """Our tcgen05 attention backward (csrc/attn_bwd_sm100.cu): pre-pass (row statistics, zero dQ accumulator), main
     kernel, post-pass (dQ fp32 -> bf16).  With ``dqkv`` the three gradients land in the column blocks of that packed
     [T, (Hq+2*Hkv)*D] buffer (returned); otherwise returns dense (dq, dk, dv).  With ``cos``/``sin`` the post-pass also
-    undoes the RoPE rotation of dq and dk (the backward of the fused QKV+RoPE projection epilogue)."""
+    undoes the RoPE rotation of dq and dk (the backward of the fused QKV+RoPE projection epilogue).  ``mask``: the
+    MASKED kernel instantiation."""
     assert D == 64 and S % 128 == 0 and dout.is_contiguous() and out.is_contiguous()
     T = B * S
     dev = qkv.device
-    dq_acc, stats = _bwd_scratch(dev, T, Hq, D)
+    dq_acc, stats = _bwd_scratch(dev, T, Hq, D, masked=mask is not None)
     if dqkv is not None:
         dq, dk, dv = dqkv[:, : Hq * D], dqkv[:, Hq * D:(Hq + Hkv) * D], dqkv[:, (Hq + Hkv) * D:]
     else:
@@ -73,20 +120,31 @@ def tc_attention_bwd(dout: torch.Tensor, qkv: torch.Tensor, out: torch.Tensor, l
         dk = torch.empty(T, Hkv * D, dtype=qkv.dtype, device=dev)
         dv = torch.empty(T, Hkv * D, dtype=qkv.dtype, device=dev)
     assert dk.stride(0) == dv.stride(0)
-    _lib.check(_lib.cuda_lib().odb_attn_bwd(qkv.data_ptr(), out.data_ptr(), dout.data_ptr(), lse.data_ptr(), stats.data_ptr(),
-                                            dq_acc.data_ptr(), dq.data_ptr(), dk.data_ptr(), dv.data_ptr(),
-                                            cos.data_ptr() if cos is not None else None, sin.data_ptr() if sin is not None else None,
-                                            B, S, Hq, Hkv, qkv.stride(0), out.stride(0), dq.stride(0), dk.stride(0),
-                                            1.0 / math.sqrt(D), _lib.stream_ptr(qkv)), "attn_bwd")
+    args = (qkv.data_ptr(), out.data_ptr(), dout.data_ptr(), lse.data_ptr(), stats.data_ptr(), dq_acc.data_ptr(), dq.data_ptr(),
+            dk.data_ptr(), dv.data_ptr(), cos.data_ptr() if cos is not None else None, sin.data_ptr() if sin is not None else None,
+            B, S, Hq, Hkv, qkv.stride(0), out.stride(0), dq.stride(0), dk.stride(0), 1.0 / math.sqrt(D))
+    if mask is None:
+        _lib.check(_lib.cuda_lib().odb_attn_bwd(*args, _lib.stream_ptr(qkv)), "attn_bwd")
+    else:
+        _lib.check(_lib.cuda_lib().odb_attn_bwd_masked(*args, mask.lo.data_ptr(), mask.vbits.data_ptr(), mask.q_hi.data_ptr(),
+                                                       mask.lo_hi.data_ptr(), _lib.stream_ptr(qkv)), "attn_bwd_masked")
     _lib.count_launch(3)
     return dqkv if dqkv is not None else (dq, dk, dv)
 
 
-def tc_attention_fwd(qkv: torch.Tensor, B: int, S: int, Hq: int, Hkv: int, D: int = 64, dbg: torch.Tensor | None = None):
-    """Our tcgen05 causal attention forward.  Returns (out [T, Hq*D] bf16, lse [B, Hq, S] fp32, natural log)."""
+def tc_attention_fwd(qkv: torch.Tensor, B: int, S: int, Hq: int, Hkv: int, D: int = 64, dbg: torch.Tensor | None = None,
+                     mask: MaskDesc | None = None):
+    """Our tcgen05 causal attention forward.  Returns (out [T, Hq*D] bf16, lse [B, Hq, S] fp32, natural log).
+    ``mask``: the MASKED kernel instantiation."""
     assert D == 64 and S % 128 == 0 and qkv.dtype == torch.bfloat16 and qkv.stride(1) == 1
     out = torch.empty(B * S, Hq * D, dtype=qkv.dtype, device=qkv.device)
     lse = torch.empty(B, Hq, S, dtype=torch.float32, device=qkv.device)
+    if mask is not None:
+        _lib.check(_lib.cuda_lib().odb_attn_fwd_masked(qkv.data_ptr(), out.data_ptr(), lse.data_ptr(), B, S, Hq, Hkv, qkv.stride(0),
+                                                       out.stride(0), 1.0 / math.sqrt(D), mask.lo.data_ptr(), mask.vbits.data_ptr(),
+                                                       mask.kv_lo.data_ptr(), _lib.stream_ptr(qkv)), "attn_fwd_masked")
+        _lib.count_launch()
+        return out, lse
     _lib.check(_lib.cuda_lib().odb_attn_fwd(qkv.data_ptr(), out.data_ptr(), lse.data_ptr(), B, S, Hq, Hkv, qkv.stride(0),
                                             out.stride(0), 1.0 / math.sqrt(D), dbg.data_ptr() if dbg is not None else None,
                                             _lib.stream_ptr(qkv)), "attn_fwd")
@@ -113,10 +171,29 @@ def split_qkv(qkv: torch.Tensor, B: int, S: int, Hq: int, Hkv: int, D: int):
     return q, k, v
 
 
-def attention_fwd(qkv: torch.Tensor, B: int, S: int, Hq: int, Hkv: int, D: int):
-    """Returns (out [T, Hq*D], lse).  Causal, scale 1/sqrt(D)."""
+def _sdpa_masked_fwd(qkv, mask: MaskDesc, B, S, Hq, Hkv, D):
+    """CUDA fallback of the masked cases the tcgen05 kernels do not take: torch SDPA with the dense mask, differentiated
+    by autograd in ``attention_bwd``."""
+    q, k, v = split_qkv(qkv, B, S, Hq, Hkv, D)
+    leaves = [t.detach().transpose(1, 2).requires_grad_(True) for t in (q, k, v)]
+    with torch.enable_grad():
+        o = torch.nn.functional.scaled_dot_product_attention(leaves[0], leaves[1], leaves[2], attn_mask=dense_mask(mask, B, S),
+                                                             enable_gqa=(Hq != Hkv))
+        out = o.transpose(1, 2).reshape(B * S, Hq * D)
+    return out.detach(), ("sdpa", out, leaves)
+
+
+def attention_fwd(qkv: torch.Tensor, B: int, S: int, Hq: int, Hkv: int, D: int, mask: MaskDesc | None = None):
+    """Returns (out [T, Hq*D], aux).  Causal, scale 1/sqrt(D); ``mask`` restricts it further (see ``MaskDesc``)."""
     q, k, v = split_qkv(qkv, B, S, Hq, Hkv, D)
     scale = 1.0 / math.sqrt(D)
+    if mask is not None and qkv.is_cuda:
+        if _LIB == "tc" and _tc_usable(qkv, S, Hq, Hkv, D):
+            if not (_lib.has_symbol("odb_attn_fwd_masked") and _lib.has_symbol("odb_attn_bwd_masked")):
+                raise _lib.NativeLibraryMissing("libodb200.so lacks the masked attention kernels: rebuild it")
+            out, lse = tc_attention_fwd(qkv, B, S, Hq, Hkv, D, mask=mask)
+            return out, ("tc", lse)
+        return _sdpa_masked_fwd(qkv, mask, B, S, Hq, Hkv, D)
     if qkv.is_cuda and qkv.dtype in (torch.bfloat16, torch.float16):
         if _LIB == "tc" and _tc_usable(qkv, S, Hq, Hkv, D):
             out, lse = tc_attention_fwd(qkv, B, S, Hq, Hkv, D)
@@ -136,8 +213,8 @@ def attention_fwd(qkv: torch.Tensor, B: int, S: int, Hq: int, Hkv: int, D: int):
         rep = Hq // Hkv
         kf, vf = kf.repeat_interleave(rep, dim=1), vf.repeat_interleave(rep, dim=1)
     att = (qf @ kf.transpose(-1, -2)) * scale
-    mask = torch.ones(S, S, dtype=torch.bool, device=qkv.device).tril()
-    att = att.masked_fill(~mask, float("-inf"))
+    allowed = torch.ones(S, S, dtype=torch.bool, device=qkv.device).tril() if mask is None else dense_mask(mask, B, S)
+    att = att.masked_fill(~allowed, float("-inf"))
     lse = torch.logsumexp(att, dim=-1)
     p = torch.softmax(att, dim=-1)
     out = (p @ vf).permute(0, 2, 1, 3).reshape(B * S, Hq * D).to(qkv.dtype)
@@ -145,13 +222,21 @@ def attention_fwd(qkv: torch.Tensor, B: int, S: int, Hq: int, Hkv: int, D: int):
 
 
 def attention_bwd(dout: torch.Tensor, qkv: torch.Tensor, out: torch.Tensor, aux, dqkv: torch.Tensor, B: int, S: int,
-                  Hq: int, Hkv: int, D: int, want_parts: bool = False, rope=None):
+                  Hq: int, Hkv: int, D: int, want_parts: bool = False, rope=None, mask: MaskDesc | None = None):
     """Writes dq|dk|dv into the packed ``dqkv`` buffer (same layout as qkv) and returns it - or, with ``want_parts`` and a
     back-end that produces separate dense gradients, returns the tuple (dq [T,Hq*D], dk [T,Hkv*D], dv [T,Hkv*D]).
-    ``rope=(cos, sin)``: a back-end for which ``bwd_applies_rope(aux)`` holds also undoes the rotation of dq / dk."""
+    ``rope=(cos, sin)``: a back-end for which ``bwd_applies_rope(aux)`` holds also undoes the rotation of dq / dk.
+    ``mask``: the description the forward ran with."""
     if isinstance(aux[0], str) and aux[0] == "tc":
         cos, sin = rope if rope is not None else (None, None)
-        return tc_attention_bwd(dout, qkv, out, aux[1], B, S, Hq, Hkv, D, dqkv=dqkv, cos=cos, sin=sin)
+        return tc_attention_bwd(dout, qkv, out, aux[1], B, S, Hq, Hkv, D, dqkv=dqkv, cos=cos, sin=sin, mask=mask)
+    if isinstance(aux[0], str) and aux[0] == "sdpa":
+        gq, gk, gv = torch.autograd.grad(aux[1], aux[2], dout)
+        dq, dk, dv = split_qkv(dqkv, B, S, Hq, Hkv, D)
+        dq.copy_(gq.transpose(1, 2))
+        dk.copy_(gk.transpose(1, 2))
+        dv.copy_(gv.transpose(1, 2))
+        return dqkv
     q, k, v = split_qkv(qkv, B, S, Hq, Hkv, D)
     dq, dk, dv = split_qkv(dqkv, B, S, Hq, Hkv, D)
     scale = 1.0 / math.sqrt(D)
@@ -180,8 +265,8 @@ def attention_bwd(dout: torch.Tensor, qkv: torch.Tensor, out: torch.Tensor, aux,
     if rep != 1:
         kf, vf = kf.repeat_interleave(rep, dim=1), vf.repeat_interleave(rep, dim=1)
     att = (qf @ kf.transpose(-1, -2)) * scale
-    mask = torch.ones(S, S, dtype=torch.bool, device=qkv.device).tril()
-    att = att.masked_fill(~mask, float("-inf"))
+    allowed = torch.ones(S, S, dtype=torch.bool, device=qkv.device).tril() if mask is None else dense_mask(mask, B, S)
+    att = att.masked_fill(~allowed, float("-inf"))
     p = torch.softmax(att, dim=-1)
     do = dout.float().view(B, S, Hq, D).permute(0, 2, 1, 3)
     dvf = p.transpose(-1, -2) @ do

@@ -399,3 +399,57 @@ def nesterov_outer(theta_outer: torch.Tensor, buf: torch.Tensor, delta: torch.Te
     theta_local.copy_(theta_outer)
     if shadow is not None:
         shadow.copy_(theta_outer)
+
+
+# ------------------------------------------------------------------------------------------------ attention mask description
+_lib.register_optional("odb_attn_mask_prep", [_ct.c_void_p, _ct.c_void_p, _ct.c_int, _ct.c_int, _ct.c_int, _ct.c_longlong]
+                       + [_ct.c_void_p] * 6)
+
+
+def attn_mask_prep(ids: torch.Tensor, mask: torch.Tensor | None, eos: int, lo: torch.Tensor, vbits: torch.Tensor,
+                   kv_lo: torch.Tensor, q_hi: torch.Tensor, lo_hi: torch.Tensor) -> None:
+    """Compact description of a padding and/or per-document causal mask (outputs int32, written in place).
+
+    For row b, query s and key t: ``valid[t] = mask[b, t] != 0`` (all ones without a mask); ``docstart[s]`` = 0, or 1 + the
+    last p < s with ``ids[b, p] == eos`` (``eos < 0``: no document masking); ``lo[s] = min(s, first t >= docstart[s] with
+    valid[t])``; attention is allowed where ``t == s or (lo[s] <= t < s and valid[t])``.
+
+    lo [B*S]; vbits [B, ceil(S/32)] (bit t%32 of word t//32 = valid[t]); per 128-query tile qt: kv_lo = min lo // 128 and
+    lo_hi = max lo; per 128-key tile kt: q_hi = max{qt : kv_lo[qt] <= kt}.  ids int64 [B, S]; mask [B, S] of any integer
+    or bool dtype."""
+    B, S = ids.shape
+    if ids.is_cuda:
+        assert ids.dtype == torch.int64 and ids.is_contiguous()
+        assert mask is None or (mask.shape == ids.shape and mask.is_contiguous() and mask.device == ids.device)
+        for t in (lo, vbits, kv_lo, q_hi, lo_hi):
+            assert t.dtype == torch.int32 and t.is_contiguous()
+        _lib.check(_lib.cuda_lib().odb_attn_mask_prep(_p(ids), _p(mask), mask.element_size() if mask is not None else 0, B, S,
+                                                      int(eos), _p(lo), _p(vbits), _p(kv_lo), _p(q_hi), _p(lo_hi),
+                                                      _lib.stream_ptr(ids)), "attn_mask_prep")
+        _lib.count_launch()
+        return
+    dev = ids.device
+    pos = torch.arange(S, device=dev)
+    valid = torch.ones(B, S, dtype=torch.bool, device=dev) if mask is None else (mask != 0)
+    if eos >= 0:
+        after = torch.where(ids == eos, pos + 1, 0).cummax(dim=1).values      # 1 + last EOS at or before p
+        docstart = torch.cat([torch.zeros(B, 1, dtype=after.dtype, device=dev), after[:, :-1]], dim=1)
+    else:
+        docstart = torch.zeros(B, S, dtype=torch.int64, device=dev)
+    nv = torch.where(valid, pos, S).flip(1).cummin(dim=1).values.flip(1)     # first valid position >= p
+    l = torch.minimum(pos[None], nv.gather(1, docstart))
+    lo.copy_(l.reshape(-1))
+    nw, nq = (S + 31) // 32, (S + 127) // 128
+    vb = torch.zeros(B, nw * 32, dtype=torch.int64, device=dev)
+    vb[:, :S] = valid.long()
+    w = (vb.view(B, nw, 32) << torch.arange(32, device=dev)).sum(-1)
+    vbits.copy_(torch.where(w >= 2 ** 31, w - 2 ** 32, w))
+    lp = torch.full((B, nq * 128), S, dtype=torch.int64, device=dev)
+    lp[:, :S] = l
+    kmin = lp.view(B, nq, 128).amin(-1)
+    lp[:, S:] = -1
+    lo_hi.copy_(lp.view(B, nq, 128).amax(-1))
+    kv_lo.copy_(kmin // 128)
+    tiles = torch.arange(nq, device=dev)
+    reach = (kmin // 128)[:, None, :] <= tiles[None, :, None]                 # [B, kt, qt]
+    q_hi.copy_(torch.where(reach, tiles[None, None, :], -1).amax(-1))

@@ -65,6 +65,8 @@ class TorchDilocoConfig(BaseConfig):
     fake_data: bool = False
     token_shards: str | None = None         # glob of pre-tokenised shards (scripts/tokenize_corpus.py) instead of streaming C4
     eval_token_shards: str | None = None
+    # attention stays inside the EOS-terminated documents of a packed row (token shards concatenate documents)
+    document_mask: bool = False
     max_steps: int | None = None
     metric_logger_type: Literal["wandb", "dummy"] = "wandb"
     seed: int = 0
@@ -111,14 +113,15 @@ def load_checkpoint(model, optimizer: DiLoCoOptimizer, scheduler, filename: str,
 
 
 @torch.no_grad()
-def evaluate_model(eval_loader, model, max_batches: int) -> dict:
+def evaluate_model(eval_loader, model, max_batches: int, document_mask: bool = False) -> dict:
     """Mean eval loss / perplexity (reference train_diloco_torch.py:87-110; unlike the reference the eval runs in the
     training precision instead of hard-coded fp16 autocast - SURVEY.md §2.7)."""
     model.eval()
     t0, tot, n = time.time(), 0.0, 0
     for batch in eval_loader:
         dev = model.device
-        out = model(input_ids=batch["input_ids"].to(dev), attention_mask=batch.get("attention_mask"), labels=batch["labels"].to(dev))
+        out = model(input_ids=batch["input_ids"].to(dev), attention_mask=batch.get("attention_mask"), labels=batch["labels"].to(dev),
+                    document_mask=document_mask)
         tot += float(out.loss)
         n += 1
         if n >= max_batches:
@@ -195,9 +198,11 @@ def main(cfg: TorchDilocoConfig) -> None:
             handles = register_metrics_hooks(model, ["self_attn", "lm_head"], log_activations, grad_accum)
         ids, labels = batch["input_ids"].to(device, non_blocking=True), batch["labels"].to(device, non_blocking=True)
         if native:
-            loss = model.forward_backward(ids, labels, 1.0 / grad_accum, batch.get("attention_mask")) / grad_accum
+            loss = model.forward_backward(ids, labels, 1.0 / grad_accum, batch.get("attention_mask"),
+                                          document_mask=cfg.document_mask) / grad_accum
         else:
-            loss = model(input_ids=ids, attention_mask=batch.get("attention_mask"), labels=labels).loss / grad_accum
+            loss = model(input_ids=ids, attention_mask=batch.get("attention_mask"), labels=labels,
+                         document_mask=cfg.document_mask).loss / grad_accum
             scaler.scale(loss).backward()
         loss_batch += loss.detach()
         if not boundary:
@@ -218,7 +223,7 @@ def main(cfg: TorchDilocoConfig) -> None:
 
         eval_metrics = {}
         if rank == 0 and cfg.eval_steps is not None and real_step % cfg.eval_steps == 0:
-            eval_metrics = evaluate_model(eval_loader, model, cfg.eval_batches)
+            eval_metrics = evaluate_model(eval_loader, model, cfg.eval_batches, cfg.document_mask)
         if rank == 0:
             lv = float(loss_batch.item())
             m = {"Loss": lv, "step": real_step, "lr": inner.param_groups[0]["lr"], "Perplexity": math.exp(min(lv, 50)),

@@ -103,6 +103,8 @@ class Config(BaseConfig):
     # DiLoCo ("hv" kept as the flag namespace of the reference)
     hv: HvConfig | None = None
     fake_data: bool = False
+    # attention stays inside the EOS-terminated documents of a packed row (tokens: shards concatenate documents)
+    document_mask: bool = False
     max_steps: int | None = None
     seed: int = 0
 
@@ -229,9 +231,9 @@ def train(config: Config) -> None:
         labels = batch["labels"].to(device, non_blocking=True)
         mask = batch.get("attention_mask")
         if use_native:
-            loss = model.forward_backward(ids, labels, 1.0 / grad_accum, mask) / grad_accum
+            loss = model.forward_backward(ids, labels, 1.0 / grad_accum, mask, document_mask=config.document_mask) / grad_accum
         else:   # fp16: loss scaling goes through autograd + GradScaler exactly like the reference (train_fsdp.py:378-383)
-            loss = model(input_ids=ids, attention_mask=mask, labels=labels).loss / grad_accum
+            loss = model(input_ids=ids, attention_mask=mask, labels=labels, document_mask=config.document_mask).loss / grad_accum
             scaler.scale(loss).backward()
         loss_batch += loss.detach()
         for h in handles:
