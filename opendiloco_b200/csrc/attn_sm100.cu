@@ -1,4 +1,4 @@
-// Causal flash-attention forward on tcgen05 / TMEM / TMA for sm_100a (SURVEY.md §2.5 K5), head_dim 64, bf16, MHA + GQA.
+// Causal flash-attention forward on tcgen05 / TMEM / TMA for sm_100a (SURVEY.md §2.5 K5), head_dim 64 or 128, bf16, MHA + GQA.
 //
 // Reads q/k/v straight out of the packed projection buffer qkv[T, (Hq + 2*Hkv) * 64] (token-major rows: no transposes)
 // through ONE tensor map, writes out[T, Hq*64] token-major (the o-proj GEMM's A operand) and lse[B, Hq, S].
@@ -12,6 +12,10 @@
 //              64-127, row max exchanged through shared memory): tcgen05.ld S, online max/sum with exp2, causal mask
 //              on the diagonal tile, rescale O in TMEM (tcgen05.ld/st), write P (bf16) into the swizzled smem operand;
 //              epilogue: O / l -> bf16 -> swizzled staging tile -> TMA store
+//
+// Head size 128 (template parameter D): every [128 x D] operand is two 64-column TMA boxes, QK^T takes eight K16 steps
+// across them, PV is N = 128 with V's two boxes as its MN chunks, and the softmax threads rescale / store 64 O columns
+// each.  160 KB of shared memory and 320 TMEM columns (allocated 512) leave room for one CTA per SM only.
 //
 // MASKED instantiation (padding / per-document masks, described by odb_attn_mask_prep below): every role walks key tiles
 // kv_lo[b, qt] .. qt instead of 0 .. qt; a warp whose rows see only allowed keys in a tile takes the causal code, the
@@ -28,16 +32,24 @@ using namespace packed_math;
 
 namespace attn {
 
-constexpr int BQ = 128, BKV = 128, D = 64;
-constexpr int TILE_BYTES = 128 * 128;           // a [128 x 64] bf16 tile (128-byte rows)
+constexpr int BQ = 128, BKV = 128;
+constexpr int TILE_BYTES = 128 * 128;           // a [128 x 64] bf16 box (128-byte rows); a [128 x D] operand is D/64 boxes
 constexpr int THREADS = 320;
 constexpr int SOFTMAX_THREADS = 256;
-// 7 tiles + barriers = 114,816 B: two CTAs per SM need 2 x (smem + 1 KB reserved) <= 227 KB, so there is no slack for a
-// manual 1024-byte round-up - the dynamic window is declared 1024-aligned instead (it starts at the CTA's smem base)
-constexpr int SMEM_BYTES = TILE_BYTES /*Q*/ + 2 * TILE_BYTES /*K x2*/ + TILE_BYTES /*V x1*/ + TILE_BYTES /*out staging*/ + 128 /*barriers*/;   // 82 KB + 2 KB static
-// the row-max / row-sum exchange between the two column halves lives in the (otherwise unused) tail of the barrier block
-// plus a small static array
-constexpr uint32_t TMEM_COLS = 256;             // S: [0,128)  O: [128,192)  P (bf16, 2 keys per column): [192,256)
+// Per head size D (64 or 128):
+//   D = 64 : 7 boxes + barriers = 114,816 B: two CTAs per SM need 2 x (smem + 1 KB reserved) <= 227 KB, so there is no slack
+//            for a manual 1024-byte round-up - the dynamic window is declared 1024-aligned instead (it starts at the CTA's
+//            smem base).  TMEM 256 columns - S: [0,128)  O: [128,192)  P (bf16, 2 keys per column): [192,256)
+//   D = 128: 14 boxes (Q 2, K 2 x 2, V 2, out staging 2) = 160 KB: one CTA per SM.  S 128 + O 128 + P 64 = 320 columns, so
+//            the allocation is 512 - S: [0,128)  O: [128,256)  P: [256,320)
+template <int D> struct FwdCfg {
+  static_assert(D == 64 || D == 128, "head size");
+  static constexpr int NB = D / 64;             // 64-column boxes per [128 x D] operand
+  static constexpr int OP_BYTES = NB * TILE_BYTES;
+  static constexpr int SMEM_BYTES = OP_BYTES /*Q*/ + 2 * OP_BYTES /*K x2*/ + OP_BYTES /*V x1*/ + OP_BYTES /*out staging*/ + 128 /*barriers*/;
+  static constexpr uint32_t TMEM_COLS = D == 64 ? 256 : 512;
+  static constexpr int MIN_BLOCKS = D == 64 ? 2 : 1;
+};
 
 struct Params {
   int B, S, Hq, Hkv;
@@ -52,17 +64,19 @@ struct Params {
 
 #define ATT_STAMP(slot) do { if (dbg_on) p.dbg[j * 16 + (slot)] = clock64(); } while (0)
 
-template <bool MASKED>
-__global__ void __launch_bounds__(THREADS, 2)
+template <bool MASKED, int D = 64>
+__global__ void __launch_bounds__(THREADS, FwdCfg<D>::MIN_BLOCKS)
 attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_constant__ CUtensorMap tmap_out, Params p) {
+  constexpr int NB = FwdCfg<D>::NB, OP_BYTES = FwdCfg<D>::OP_BYTES;
+  constexpr uint32_t TMEM_COLS = FwdCfg<D>::TMEM_COLS;
   extern __shared__ __align__(1024) uint8_t smem[];
   __shared__ float red[2 * 256];                 // row max / row sum exchange between the two column halves (double-buffered)
   if (threadIdx.x == 0 && (smem_u32(smem) & 1023u)) __trap();     // swizzled tiles need 1024-byte alignment
   uint8_t* sQ = smem;
-  uint8_t* sK = sQ + TILE_BYTES;
-  uint8_t* sV = sK + 2 * TILE_BYTES;            // single V stage: V_{j+1} is only needed after softmax_{j+1}
-  uint8_t* sOut = sV + TILE_BYTES;              // output staging tile (P lives in tensor memory)
-  uint64_t* q_full = reinterpret_cast<uint64_t*>(sOut + TILE_BYTES);
+  uint8_t* sK = sQ + OP_BYTES;
+  uint8_t* sV = sK + 2 * OP_BYTES;              // single V stage: V_{j+1} is only needed after softmax_{j+1}
+  uint8_t* sOut = sV + OP_BYTES;                // output staging tile (P lives in tensor memory)
+  uint64_t* q_full = reinterpret_cast<uint64_t*>(sOut + OP_BYTES);
   uint64_t* k_full = q_full + 1;                // [2]
   uint64_t* k_empty = k_full + 2;               // [2]
   uint64_t* v_full = k_empty + 2;
@@ -106,7 +120,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
   __syncthreads();
   tc_fence_after_sync();
   const uint32_t tmem_base = *tmem_slot;
-  const uint32_t tS = tmem_base, tO = tmem_base + 128, tP = tmem_base + 192;
+  const uint32_t tS = tmem_base, tO = tmem_base + 128, tP = tmem_base + 128 + D;
   pdl_wait();
 
   if (warp == 0) {
@@ -116,34 +130,40 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
       auto load_k = [&](int j, int tg) {
         const int st = tg & 1;
         mbar_wait(&k_empty[st], ((tg >> 1) & 1) ^ 1);
-        mbar_arrive_expect_tx(&k_full[st], TILE_BYTES);
-        tma_load_2d(sK + st * TILE_BYTES, &tmap_qkv, &k_full[st], col_k, b * p.S + j * BKV);
+        mbar_arrive_expect_tx(&k_full[st], OP_BYTES);
+#pragma unroll
+        for (int c = 0; c < NB; ++c)
+          tma_load_2d(sK + st * OP_BYTES + c * TILE_BYTES, &tmap_qkv, &k_full[st], col_k + 64 * c, b * p.S + j * BKV);
       };
       for (int w = 0, t0 = 0; w < nitems; ++w) {
         const int j0 = MASKED ? p.kv_lo[b * nq + qb[w]] : 0;
         const int nkv = qb[w] + 1 - j0;          // causal: key tiles j0..qblk
         mbar_wait(q_empty, (w & 1) ^ 1);
-        mbar_arrive_expect_tx(q_full, TILE_BYTES);
-        tma_load_2d(sQ, &tmap_qkv, q_full, col_q, b * p.S + qb[w] * BQ);
+        mbar_arrive_expect_tx(q_full, OP_BYTES);
+#pragma unroll
+        for (int c = 0; c < NB; ++c) tma_load_2d(sQ + c * TILE_BYTES, &tmap_qkv, q_full, col_q + 64 * c, b * p.S + qb[w] * BQ);
         load_k(j0, t0);
         for (int j = 0; j < nkv; ++j) {
           const int tg = t0 + j;
           if (j + 1 < nkv) load_k(j0 + j + 1, tg + 1);
           mbar_wait(v_empty, (tg & 1) ^ 1);
-          mbar_arrive_expect_tx(v_full, TILE_BYTES);
-          tma_load_2d(sV, &tmap_qkv, v_full, col_v, b * p.S + (j0 + j) * BKV);
+          mbar_arrive_expect_tx(v_full, OP_BYTES);
+#pragma unroll
+          for (int c = 0; c < NB; ++c)
+            tma_load_2d(sV + c * TILE_BYTES, &tmap_qkv, v_full, col_v + 64 * c, b * p.S + (j0 + j) * BKV);
         }
         t0 += nkv;
       }
     }
   } else if (warp == 1) {
     constexpr uint32_t idesc_qk = make_idesc_bf16(BQ, BKV, 0, 0);   // S[128,128] = Q (K-major) x K^T (K-major)
-    constexpr uint32_t idesc_pv = make_idesc_bf16(BQ, D, 0, 1);     // O[128,64] = P (TMEM, K-major) x V (smem, MN-major)
+    constexpr uint32_t idesc_pv = make_idesc_bf16(BQ, D, 0, 1);     // O[128,D] = P (TMEM, K-major) x V (smem, MN-major)
     const bool leader = elect_one();             // the same lane issues every MMA / commit of this CTA
     const uint64_t qd = make_smem_desc_sw128(smem_u32(sQ), 16, 1024);
-    const uint64_t vd = make_smem_desc_sw128(smem_u32(sV), 16, 1024);
+    // V read MN-major: at D = 128 its two 64-column boxes are the two MN chunks, one box (LBO) apart
+    const uint64_t vd = make_smem_desc_sw128(smem_u32(sV), NB > 1 ? TILE_BYTES : 16, 1024);
     const uint64_t kd0 = make_smem_desc_sw128(smem_u32(sK), 16, 1024);
-    const uint64_t kd1 = make_smem_desc_sw128(smem_u32(sK + TILE_BYTES), 16, 1024);
+    const uint64_t kd1 = make_smem_desc_sw128(smem_u32(sK + OP_BYTES), 16, 1024);
     const bool dbg_cta = p.dbg != nullptr && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && lane == 0;
     auto issue_qk = [&](int tg, bool last) {
       const int st = tg & 1;
@@ -155,6 +175,12 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
         umma_ss(tS, qd + 2, kd + 2, idesc_qk, 1u);
         umma_ss(tS, qd + 4, kd + 4, idesc_qk, 1u);
         umma_ss(tS, qd + 6, kd + 6, idesc_qk, 1u);
+        // D = 128: the second 64-column box of Q and K (descriptor addresses count 16-byte units)
+#pragma unroll
+        for (int k = 4; k < 4 * NB; ++k) {
+          const uint32_t o = (k / 4) * (TILE_BYTES >> 4) + 2 * (k % 4);
+          umma_ss(tS, qd + o, kd + o, idesc_qk, 1u);
+        }
         umma_commit(s_full);
         umma_commit(&k_empty[st]);               // K stage reusable once this QK retired
         if (last) umma_commit(q_empty);          // ... and so is Q after the tile's last QK
@@ -198,7 +224,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
     // ------------------------------------------------------------------ softmax / correction / epilogue
     const int q = warp & 3;
     const int row = q * 32 + lane;               // query row inside the tile == TMEM lane
-    const int half = (warp - 2) >> 2;            // 0: keys [0,64) of every tile and O columns [0,32) ; 1: the other halves
+    const int half = (warp - 2) >> 2;            // 0: keys [0,64) of every tile and O columns [0,D/2) ; 1: the other halves
     const uint32_t lane_off = (uint32_t)(q * 32) << 16;
     const float c = p.scale_log2;
     const bool dbg_cta = p.dbg != nullptr && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && threadIdx.x == 64;
@@ -300,14 +326,17 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
       if (j > 0) {
         mbar_wait(o_done, (tg - 1) & 1);         // PV_{j-1} retired: O is stable, P may be overwritten
         tc_fence_after_sync();
-        // rescale this thread's 32 columns of the running output - skipped when no row of the warp moved its reference max
+        // rescale this thread's D/2 columns of the running output - skipped when no row of the warp moved its reference max
         if (!__all_sync(0xffffffffu, alpha == 1.f)) {
-          uint32_t r[32];
-          tmem_ld_32x32b_x32(tO + lane_off + half * 32, r);
-          tmem_ld_wait();
 #pragma unroll
-          for (int i = 0; i < 32; ++i) r[i] = __float_as_uint(__uint_as_float(r[i]) * alpha);
-          tmem_st_32x32b_x32(tO + lane_off + half * 32, r);
+          for (int c = 0; c < NB; ++c) {
+            uint32_t r[32];
+            tmem_ld_32x32b_x32(tO + lane_off + half * (D / 2) + 32 * c, r);
+            tmem_ld_wait();
+#pragma unroll
+            for (int i = 0; i < 32; ++i) r[i] = __float_as_uint(__uint_as_float(r[i]) * alpha);
+            tmem_st_32x32b_x32(tO + lane_off + half * (D / 2) + 32 * c, r);
+          }
         }
       }
       ATT_STAMP(5);
@@ -329,22 +358,28 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
     mbar_wait(o_done, (t0 - 1) & 1);
     tc_fence_after_sync();
     const float inv_l = 1.f / l;
-    uint32_t r[32];
-    tmem_ld_32x32b_x32(tO + lane_off + half * 32, r);
-    tmem_ld_wait();
     uint8_t* stg = sOut;
 #pragma unroll
-    for (int u = 0; u < 4; ++u) {
-      float f[8];
+    for (int c = 0; c < NB; ++c) {
+      // this thread's columns half*D/2 + 32c .. +32: D = 64 - box 0, 16-byte units half*4 + u; D = 128 - box half, units 4c + u
+      uint32_t r[32];
+      tmem_ld_32x32b_x32(tO + lane_off + half * (D / 2) + 32 * c, r);
+      tmem_ld_wait();
 #pragma unroll
-      for (int i = 0; i < 8; ++i) f[i] = __uint_as_float(r[u * 8 + i]) * inv_l;
-      *reinterpret_cast<uint4*>(stg + row * 128 + (((half * 4 + u) ^ (row & 7)) * 16)) = pack8(f);
+      for (int u = 0; u < 4; ++u) {
+        const int box = NB > 1 ? half : 0, unit = NB > 1 ? 4 * c + u : half * 4 + u;
+        float f[8];
+#pragma unroll
+        for (int i = 0; i < 8; ++i) f[i] = __uint_as_float(r[u * 8 + i]) * inv_l;
+        *reinterpret_cast<uint4*>(stg + box * TILE_BYTES + row * 128 + ((unit ^ (row & 7)) * 16)) = pack8(f);
+      }
     }
     if (half == 0) p.lse[((size_t)b * p.Hq + h) * p.S + qblk * BQ + row] = (m * c + log2f(l)) * 0.6931471805599453f;
     fence_proxy_async_smem();
     named_bar_sync(1, SOFTMAX_THREADS);
     if (threadIdx.x == 64) {
-      tma_store_2d(&tmap_out, stg, col_q, row0);
+#pragma unroll
+      for (int c = 0; c < NB; ++c) tma_store_2d(&tmap_out, stg + c * TILE_BYTES, col_q + 64 * c, row0);
       tma_store_commit();
       tma_store_wait<0>();
     }
@@ -462,10 +497,11 @@ __global__ void __launch_bounds__(PREP_THREADS) attn_mask_prep_kernel(const long
 }  // namespace attn
 
 namespace {
-template <bool MASKED>
+template <bool MASKED, int D>
 int launch_attn_fwd(const void* qkv, void* out, void* lse, int B, int S, int Hq, int Hkv, long long ld_qkv, long long ld_out,
                     float softmax_scale, void* dbg, const int* lo, const uint32_t* vbits, const int* kv_lo, cudaStream_t st) {
   using namespace attn;
+  constexpr int SMEM_BYTES = FwdCfg<D>::SMEM_BYTES;
   if (S % BQ || Hq % Hkv || ld_qkv % 8 || ld_out % 8) return -1;
   CUtensorMap tq, to;
   int rc;
@@ -480,12 +516,12 @@ int launch_attn_fwd(const void* qkv, void* out, void* lse, int B, int S, int Hq,
   p.lo = lo; p.vbits = vbits; p.kv_lo = kv_lo;
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(attn_fwd_kernel<MASKED>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
+    cudaError_t e = cudaFuncSetAttribute(attn_fwd_kernel<MASKED, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
     if (e != cudaSuccess) return (int)e;
     attr_set = true;
   }
   dim3 grid((S / BQ + 1) / 2, Hq, B);
-  launch_pdl(attn_fwd_kernel<MASKED>, grid, dim3(THREADS), SMEM_BYTES, st, tq, to, p);
+  launch_pdl(attn_fwd_kernel<MASKED, D>, grid, dim3(THREADS), SMEM_BYTES, st, tq, to, p);
   cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? 0 : (int)e;
 }
@@ -494,7 +530,7 @@ int launch_attn_fwd(const void* qkv, void* out, void* lse, int B, int S, int Hq,
 // qkv: [B*S, (Hq+2*Hkv)*64] bf16 (row stride ld_qkv elements); out: [B*S, Hq*64] bf16; lse: [B, Hq, S] fp32
 ODB_EXPORT int odb_attn_fwd(const void* qkv, void* out, void* lse, int B, int S, int Hq, int Hkv, long long ld_qkv,
                             long long ld_out, float softmax_scale, void* dbg, cudaStream_t st) {
-  return launch_attn_fwd<false>(qkv, out, lse, B, S, Hq, Hkv, ld_qkv, ld_out, softmax_scale, dbg, nullptr, nullptr, nullptr, st);
+  return launch_attn_fwd<false, 64>(qkv, out, lse, B, S, Hq, Hkv, ld_qkv, ld_out, softmax_scale, dbg, nullptr, nullptr, nullptr, st);
 }
 
 // Same with a mask description (lo, vbits, kv_lo from odb_attn_mask_prep).
@@ -502,8 +538,22 @@ ODB_EXPORT int odb_attn_fwd_masked(const void* qkv, void* out, void* lse, int B,
                                    long long ld_out, float softmax_scale, const void* lo, const void* vbits, const void* kv_lo,
                                    cudaStream_t st) {
   if (!lo || !vbits || !kv_lo) return -1;
-  return launch_attn_fwd<true>(qkv, out, lse, B, S, Hq, Hkv, ld_qkv, ld_out, softmax_scale, nullptr, (const int*)lo,
-                               (const uint32_t*)vbits, (const int*)kv_lo, st);
+  return launch_attn_fwd<true, 64>(qkv, out, lse, B, S, Hq, Hkv, ld_qkv, ld_out, softmax_scale, nullptr, (const int*)lo,
+                                   (const uint32_t*)vbits, (const int*)kv_lo, st);
+}
+
+// Head size 128: qkv [B*S, (Hq+2*Hkv)*128], out [B*S, Hq*128]; otherwise the same arguments as odb_attn_fwd.
+ODB_EXPORT int odb_attn_fwd_d128(const void* qkv, void* out, void* lse, int B, int S, int Hq, int Hkv, long long ld_qkv,
+                                 long long ld_out, float softmax_scale, void* dbg, cudaStream_t st) {
+  return launch_attn_fwd<false, 128>(qkv, out, lse, B, S, Hq, Hkv, ld_qkv, ld_out, softmax_scale, dbg, nullptr, nullptr, nullptr, st);
+}
+
+ODB_EXPORT int odb_attn_fwd_d128_masked(const void* qkv, void* out, void* lse, int B, int S, int Hq, int Hkv, long long ld_qkv,
+                                        long long ld_out, float softmax_scale, const void* lo, const void* vbits, const void* kv_lo,
+                                        cudaStream_t st) {
+  if (!lo || !vbits || !kv_lo) return -1;
+  return launch_attn_fwd<true, 128>(qkv, out, lse, B, S, Hq, Hkv, ld_qkv, ld_out, softmax_scale, nullptr, (const int*)lo,
+                                    (const uint32_t*)vbits, (const int*)kv_lo, st);
 }
 
 // ids: int64 [B, S]; mask: optional [B, S] of any integer / bool type (mask_elem_bytes per element); eos < 0: no document

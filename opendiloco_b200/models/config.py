@@ -59,7 +59,14 @@ class LlamaConfig:
     @classmethod
     def from_dict(cls, d: dict) -> "LlamaConfig":
         known = {f for f in cls.__dataclass_fields__}
-        return cls(**{k: v for k, v in d.items() if k in known})
+        cfg = cls(**{k: v for k, v in d.items() if k in known})
+        # head_dim is derived (hidden_size / num_attention_heads: the engine's q projection is hidden_size wide); a config
+        # that asks for another head size would otherwise build a different model without a word
+        if d.get("head_dim") is not None and int(d["head_dim"]) != cfg.head_dim:
+            raise ValueError(f"head_dim {d['head_dim']} differs from hidden_size / num_attention_heads = {cfg.hidden_size} / "
+                             f"{cfg.num_attention_heads} = {cfg.head_dim}; only head_dim == hidden_size / "
+                             f"num_attention_heads is supported")
+        return cfg
 
     @classmethod
     def from_pretrained(cls, name_or_path: str) -> "LlamaConfig":

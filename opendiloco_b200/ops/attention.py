@@ -29,14 +29,22 @@ from .. import _lib
 from . import kernels as K
 
 _FLASH = None
-# Back-end of the bf16 CUDA path: "tc" = our tcgen05 kernels (csrc/attn_sm100.cu, attn_bwd_sm100.cu; head_dim 64,
-# S % 128 == 0), "cudnn" / "flash" = the library kernels (kept as comparison baselines and for other head sizes).
+# Back-end of the bf16 CUDA path: "tc" = our tcgen05 kernels (csrc/attn_sm100.cu, attn_bwd_sm100.cu,
+# attn_bwd_d128_sm100.cu; head_dim 64 or 128, S % 128 == 0), "cudnn" / "flash" = the library kernels (kept as comparison
+# baselines and for other head sizes).
 _LIB = os.environ.get("ODB_ATTN_LIB", "tc")
+
+# Entry points the tcgen05 back-end needs per head size.  A library built before the head_dim-128 kernels existed lacks
+# the second set, and such models keep the library path instead of failing.
+_TC_SYMBOLS = {
+    64: ("odb_attn_fwd", "odb_attn_bwd"),
+    128: ("odb_attn_fwd_d128", "odb_attn_bwd_d128", "odb_attn_fwd_d128_masked", "odb_attn_bwd_d128_masked"),
+}
 
 
 def _tc_usable(qkv: torch.Tensor, S: int, Hq: int, Hkv: int, D: int) -> bool:
-    return (D == 64 and S % 128 == 0 and Hq % Hkv == 0 and qkv.dtype == torch.bfloat16 and qkv.stride(1) == 1
-            and qkv.stride(0) % 8 == 0 and _lib.has_symbol("odb_attn_fwd") and _lib.has_symbol("odb_attn_bwd"))
+    return (D in _TC_SYMBOLS and S % 128 == 0 and Hq % Hkv == 0 and qkv.dtype == torch.bfloat16 and qkv.stride(1) == 1
+            and qkv.stride(0) % 8 == 0 and all(_lib.has_symbol(n) for n in _TC_SYMBOLS[D]))
 
 
 def bwd_applies_rope(aux) -> bool:
@@ -52,6 +60,17 @@ _lib.register_optional("odb_attn_fwd_masked", [ctypes.c_void_p] * 3 + [ctypes.c_
                        + [ctypes.c_float] + [ctypes.c_void_p] * 4)
 _lib.register_optional("odb_attn_bwd_masked", [ctypes.c_void_p] * 11 + [ctypes.c_int] * 4 + [ctypes.c_longlong] * 4
                        + [ctypes.c_float] + [ctypes.c_void_p] * 5)
+# head_dim 128: the forward takes the same arguments; the backward has no dQ accumulator argument and its masked form
+# also takes kv_lo (the dQ kernel walks key tiles like the forward)
+_lib.register_optional("odb_attn_fwd_d128", [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int,
+                                             ctypes.c_int, ctypes.c_int, ctypes.c_longlong, ctypes.c_longlong, ctypes.c_float,
+                                             ctypes.c_void_p, ctypes.c_void_p])
+_lib.register_optional("odb_attn_fwd_d128_masked", [ctypes.c_void_p] * 3 + [ctypes.c_int] * 4 + [ctypes.c_longlong] * 2
+                       + [ctypes.c_float] + [ctypes.c_void_p] * 4)
+_lib.register_optional("odb_attn_bwd_d128", [ctypes.c_void_p] * 10 + [ctypes.c_int] * 4 + [ctypes.c_longlong] * 4
+                       + [ctypes.c_float, ctypes.c_void_p])
+_lib.register_optional("odb_attn_bwd_d128_masked", [ctypes.c_void_p] * 10 + [ctypes.c_int] * 4 + [ctypes.c_longlong] * 4
+                       + [ctypes.c_float] + [ctypes.c_void_p] * 6)
 _SCRATCH: dict = {}
 
 
@@ -91,11 +110,12 @@ def dense_mask(desc: MaskDesc, B: int, S: int) -> torch.Tensor:
 
 def _bwd_scratch(dev, T: int, Hq: int, D: int, masked: bool = False):
     """fp32 dQ accumulator + per-query statistics of the backward kernel (reused across layers / steps: every call
-    rewrites them completely before reading).  The masked kernel keeps a third statistics row."""
+    rewrites them completely before reading).  The masked kernel keeps a third statistics row.  The head_dim-128
+    backward writes dQ once, in bf16, and needs no accumulator (None)."""
     key = (dev, T, Hq, D) if not masked else (dev, T, Hq, D, True)
     sc = _SCRATCH.get(key)
     if sc is None:
-        sc = (torch.empty(T, Hq * D, dtype=torch.float32, device=dev),
+        sc = (torch.empty(T, Hq * D, dtype=torch.float32, device=dev) if D == 64 else None,
               torch.empty((3 if masked else 2) * T * Hq, dtype=torch.float32, device=dev))
         _SCRATCH[key] = sc
     return sc
@@ -104,12 +124,12 @@ def _bwd_scratch(dev, T: int, Hq: int, D: int, masked: bool = False):
 def tc_attention_bwd(dout: torch.Tensor, qkv: torch.Tensor, out: torch.Tensor, lse: torch.Tensor, B: int, S: int, Hq: int, Hkv: int,
                      D: int = 64, dqkv: torch.Tensor | None = None, cos: torch.Tensor | None = None, sin: torch.Tensor | None = None,
                      mask: MaskDesc | None = None):
-    """Our tcgen05 attention backward (csrc/attn_bwd_sm100.cu): pre-pass (row statistics, zero dQ accumulator), main
-    kernel, post-pass (dQ fp32 -> bf16).  With ``dqkv`` the three gradients land in the column blocks of that packed
-    [T, (Hq+2*Hkv)*D] buffer (returned); otherwise returns dense (dq, dk, dv).  With ``cos``/``sin`` the post-pass also
-    undoes the RoPE rotation of dq and dk (the backward of the fused QKV+RoPE projection epilogue).  ``mask``: the
-    MASKED kernel instantiation."""
-    assert D == 64 and S % 128 == 0 and dout.is_contiguous() and out.is_contiguous()
+    """Our tcgen05 attention backward.  D = 64 (csrc/attn_bwd_sm100.cu): pre-pass (row statistics, zero dQ accumulator),
+    main kernel, post-pass (dQ fp32 -> bf16).  D = 128 (csrc/attn_bwd_d128_sm100.cu): pre-pass, dK/dV kernel, dQ kernel.
+    With ``dqkv`` the three gradients land in the column blocks of that packed [T, (Hq+2*Hkv)*D] buffer (returned);
+    otherwise returns dense (dq, dk, dv).  With ``cos``/``sin`` dq and dk also leave with the RoPE rotation undone (the
+    backward of the fused QKV+RoPE projection epilogue).  ``mask``: the MASKED kernel instantiation."""
+    assert D in (64, 128) and S % 128 == 0 and dout.is_contiguous() and out.is_contiguous()
     T = B * S
     dev = qkv.device
     dq_acc, stats = _bwd_scratch(dev, T, Hq, D, masked=mask is not None)
@@ -120,6 +140,19 @@ def tc_attention_bwd(dout: torch.Tensor, qkv: torch.Tensor, out: torch.Tensor, l
         dk = torch.empty(T, Hkv * D, dtype=qkv.dtype, device=dev)
         dv = torch.empty(T, Hkv * D, dtype=qkv.dtype, device=dev)
     assert dk.stride(0) == dv.stride(0)
+    if D == 128:
+        args = (qkv.data_ptr(), out.data_ptr(), dout.data_ptr(), lse.data_ptr(), stats.data_ptr(), dq.data_ptr(), dk.data_ptr(),
+                dv.data_ptr(), cos.data_ptr() if cos is not None else None, sin.data_ptr() if sin is not None else None,
+                B, S, Hq, Hkv, qkv.stride(0), out.stride(0), dq.stride(0), dk.stride(0), 1.0 / math.sqrt(D))
+        if mask is None:
+            _lib.check(_lib.cuda_lib().odb_attn_bwd_d128(*args, _lib.stream_ptr(qkv)), "attn_bwd_d128")
+        else:
+            _lib.check(_lib.cuda_lib().odb_attn_bwd_d128_masked(*args, mask.lo.data_ptr(), mask.vbits.data_ptr(),
+                                                                mask.kv_lo.data_ptr(), mask.q_hi.data_ptr(),
+                                                                mask.lo_hi.data_ptr(), _lib.stream_ptr(qkv)),
+                       "attn_bwd_d128_masked")
+        _lib.count_launch(3)
+        return dqkv if dqkv is not None else (dq, dk, dv)
     args = (qkv.data_ptr(), out.data_ptr(), dout.data_ptr(), lse.data_ptr(), stats.data_ptr(), dq_acc.data_ptr(), dq.data_ptr(),
             dk.data_ptr(), dv.data_ptr(), cos.data_ptr() if cos is not None else None, sin.data_ptr() if sin is not None else None,
             B, S, Hq, Hkv, qkv.stride(0), out.stride(0), dq.stride(0), dk.stride(0), 1.0 / math.sqrt(D))
@@ -136,16 +169,18 @@ def tc_attention_fwd(qkv: torch.Tensor, B: int, S: int, Hq: int, Hkv: int, D: in
                      mask: MaskDesc | None = None):
     """Our tcgen05 causal attention forward.  Returns (out [T, Hq*D] bf16, lse [B, Hq, S] fp32, natural log).
     ``mask``: the MASKED kernel instantiation."""
-    assert D == 64 and S % 128 == 0 and qkv.dtype == torch.bfloat16 and qkv.stride(1) == 1
+    assert D in (64, 128) and S % 128 == 0 and qkv.dtype == torch.bfloat16 and qkv.stride(1) == 1
     out = torch.empty(B * S, Hq * D, dtype=qkv.dtype, device=qkv.device)
     lse = torch.empty(B, Hq, S, dtype=torch.float32, device=qkv.device)
+    lib = _lib.cuda_lib()
+    fwd, fwd_masked = (lib.odb_attn_fwd, lib.odb_attn_fwd_masked) if D == 64 else (lib.odb_attn_fwd_d128, lib.odb_attn_fwd_d128_masked)
     if mask is not None:
-        _lib.check(_lib.cuda_lib().odb_attn_fwd_masked(qkv.data_ptr(), out.data_ptr(), lse.data_ptr(), B, S, Hq, Hkv, qkv.stride(0),
-                                                       out.stride(0), 1.0 / math.sqrt(D), mask.lo.data_ptr(), mask.vbits.data_ptr(),
-                                                       mask.kv_lo.data_ptr(), _lib.stream_ptr(qkv)), "attn_fwd_masked")
+        _lib.check(fwd_masked(qkv.data_ptr(), out.data_ptr(), lse.data_ptr(), B, S, Hq, Hkv, qkv.stride(0), out.stride(0),
+                              1.0 / math.sqrt(D), mask.lo.data_ptr(), mask.vbits.data_ptr(), mask.kv_lo.data_ptr(),
+                              _lib.stream_ptr(qkv)), "attn_fwd_masked")
         _lib.count_launch()
         return out, lse
-    _lib.check(_lib.cuda_lib().odb_attn_fwd(qkv.data_ptr(), out.data_ptr(), lse.data_ptr(), B, S, Hq, Hkv, qkv.stride(0),
+    _lib.check(fwd(qkv.data_ptr(), out.data_ptr(), lse.data_ptr(), B, S, Hq, Hkv, qkv.stride(0),
                                             out.stride(0), 1.0 / math.sqrt(D), dbg.data_ptr() if dbg is not None else None,
                                             _lib.stream_ptr(qkv)), "attn_fwd")
     _lib.count_launch()
